@@ -11,7 +11,7 @@ run" (north star) and "the unchanged example drivers on the GPU path" possible t
   * ``_stubs/cma.py`` and ``_stubs/matplotlib/pyplot.py`` are import stand-ins for the two packages
     ``example/inverse/_inverse.py:4,10`` imports at module top and ``solve_gd`` never touches.
 
-    python baseline/install_ref.py            # in the build container (needs /root/reference)
+    DHTS_REFERENCE=<checkout of the original project> python baseline/install_ref.py
 """
 from __future__ import annotations
 
@@ -24,7 +24,7 @@ import tempfile
 HERE = os.path.dirname(os.path.abspath(__file__))
 REF = os.path.join(HERE, "_ref")
 STUBS = os.path.join(REF, "_stubs")
-SRC = os.environ.get("DHTS_REFERENCE", "/root/reference")
+SRC = os.environ.get("DHTS_REFERENCE", "")         # a checkout of the original project
 PACKAGES = ("model", "road", "dmath", "example")
 
 
@@ -36,7 +36,7 @@ def install(force: bool = False) -> str | None:
     """Copy the reference into baseline/_ref (no-op when it is already there or the source is absent)."""
     if available() and not force:
         return REF
-    if not os.path.isdir(os.path.join(SRC, "road")):
+    if not (SRC and os.path.isdir(os.path.join(SRC, "road"))):
         return None
     os.makedirs(REF, exist_ok=True)
     for pkg in PACKAGES:

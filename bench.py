@@ -34,6 +34,8 @@ sys.path.insert(0, ROOT)
 ARZ_SCALARS_FWD, ARZ_SCALARS_BWD = 4, 6          # fwd: read (r,y) write (r,y); bwd: read (r,y), read adj, write adj
 IDM_SCALARS_FWD, IDM_SCALARS_BWD = 10, 12        # fwd: read (p,v)+6 params, write (p,v); bwd: read 8 + adj 2 + write 2
 SEED = 20221008
+# --dump-outputs: bytes for the 5 ARZ arrays of [lanes, cells] and the 4 IDM arrays of [vehicles]; 56 MB in all
+DUMP_ARZ_BYTES, DUMP_IDM_BYTES = 40 << 20, 16 << 20
 
 
 def parse():
@@ -59,7 +61,17 @@ def parse():
     ap.add_argument("--no-parity", action="store_true", help="skip the oracle check of sampled lanes")
     ap.add_argument("--no-drivers", action="store_true", help="skip configs 1-3 under the reference's unchanged drivers")
     ap.add_argument("--net-replicas", type=int, default=2048)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy in the state dtype: "
+                         "the losses, and final states and initial-state gradients of a fixed seeded sample of lanes. "
+                         "The sample is gathered on the device in the last timed step, after each rollout's closing "
+                         "event: the per-phase times and rates exclude it, ms_per_step includes those few small copies")
+    a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
+    return a
 
 
 def workload_name(a):
@@ -401,7 +413,8 @@ class Batch:
     def arz_pass(self, d, timers=None, before_chunk=None, after_chunk=None, capture=None):
         """fwd + loss + adjoint of all B lanes, chunk of lanes by chunk of lanes (lanes are independent).
         before_chunk(i) / after_chunk(i, g_r0, g_u0) let the end-to-end pass pipeline its copies with the compute;
-        capture = {"idx": LongTensor of lanes} collects rT / uT rows of those lanes (parity check)."""
+        capture = self.lane_capture(lanes) collects the rT / yT / uT / g_r0 / g_u0 rows of those lanes with device-side
+        gathers only, so that a timed pass can capture without a host synchronisation."""
         torch, F, A = self.torch, self.F, self.A
         g_r0 = torch.empty_like(d["r0"]); g_u0 = torch.empty_like(d["u0"])
         total = torch.zeros((), dtype=self.dt_t, device=self.dev)
@@ -420,14 +433,23 @@ class Batch:
             g_r0[lo:hi] = r0.grad; g_u0[lo:hi] = u0.grad
             total += loss.detach()
             if capture is not None:
-                sel = capture["idx"][(capture["idx"] >= lo) & (capture["idx"] < hi)]
-                if sel.numel():
-                    capture.setdefault("rows", []).append(sel.cpu())
-                    capture.setdefault("rT", []).append(rT.detach()[sel - lo].cpu())
-                    capture.setdefault("uT", []).append(uT.detach()[sel - lo].cpu())
+                for k, x in (("rT", rT), ("yT", yT), ("uT", uT)):
+                    capture.setdefault(k, []).append(x.detach().index_select(0, capture["rows"][ci]))
             if after_chunk: after_chunk(ci, g_r0, g_u0)
             del rT, yT, uT, loss, r0, u0
+        if capture is not None:
+            for k in ("rT", "yT", "uT"):
+                capture[k] = torch.cat(capture[k])
+            capture["g_r0"], capture["g_u0"] = (g.index_select(0, capture["lanes"]) for g in (g_r0, g_u0))
         return total, g_r0, g_u0
+
+    def lane_capture(self, lanes):
+        """Capture spec of arz_pass for the sorted lane indices `lanes`: their device indices, and per lane chunk the
+        row indices within the chunk."""
+        torch = self.torch
+        return {"lanes": torch.tensor(lanes, dtype=torch.int64, device=self.dev),
+                "rows": [torch.tensor([i - lo for i in lanes if lo <= i < hi], dtype=torch.int64, device=self.dev)
+                         for lo, hi in self.chunks]}
 
     def idm_pass(self, d, timers=None, capture=None):
         F, M = self.F, self.M
@@ -442,14 +464,15 @@ class Batch:
         loss.backward()
         if ev4: ev4[3].record(); timers.append(ev4)
         if capture is not None:
-            capture["pT"], capture["vT"] = pT.detach(), vT.detach()
+            capture["pT"], capture["vT"], capture["g_p0"], capture["g_v0"] = pT.detach(), vT.detach(), p0.grad, v0.grad
         return loss.detach(), p0.grad, v0.grad
 
     def reduce_loss(self, la, li):
         return self.shards.reduce_losses(la, li)     # the only collective: scalar losses over the lane shards
 
-    def timed(self, steps, warmup, barrier):
-        """Device-resident passes: W warm-up, then K timed, CUDA events around the whole region and around every launch."""
+    def timed(self, steps, warmup, barrier, capture=None):
+        """Device-resident passes: W warm-up, then K timed, CUDA events around the whole region and around every launch.
+        `capture` (see arz_pass) receives the outputs of the last timed pass."""
         torch = self.torch
         for _ in range(warmup):
             la, _, _ = self.arz_pass(self.devA); li, _, _ = self.idm_pass(self.devM); self.reduce_loss(la, li)
@@ -458,8 +481,10 @@ class Batch:
         tA, tM = [], []              # CUDA events (start, fwd done, loss done, bwd done) per launch pair
         e0, e1 = self.ev(), self.ev()
         e0.record()
-        for _ in range(steps):
-            la, _, _ = self.arz_pass(self.devA, tA); li, _, _ = self.idm_pass(self.devM, tM); losses = self.reduce_loss(la, li)
+        for i in range(steps):
+            cap = capture if i == steps - 1 else None
+            la, _, _ = self.arz_pass(self.devA, tA, capture=cap); li, _, _ = self.idm_pass(self.devM, tM, capture=cap)
+            losses = self.reduce_loss(la, li)
         e1.record()
         barrier()
         t_wall1 = time.time()
@@ -543,23 +568,20 @@ class Batch:
         rng = np.random.default_rng(SEED)
         idx = sorted(set([lo for lo, _ in self.chunks] + [hi - 1 for _, hi in self.chunks]
                          + [int(x) for x in rng.integers(0, self.B, 4)]))[:28]
-        cap = {"idx": torch.tensor(idx, device=self.dev)}
-        la, g_r0, g_u0 = self.arz_pass(self.devA, capture=cap)
+        cap = self.lane_capture(idx)
+        la, _, _ = self.arz_pass(self.devA, capture=cap)
         capM = {}
         li, g_p0, g_v0 = self.idm_pass(self.devM, capture=capM)
-        rows = torch.cat(cap["rows"]).numpy()
-        assert list(rows) == idx
-        rT, uT = torch.cat(cap["rT"]).numpy().astype(np.float64), torch.cat(cap["uT"]).numpy().astype(np.float64)
+        rT, uT = cap["rT"].cpu().numpy().astype(np.float64), cap["uT"].cpu().numpy().astype(np.float64)
         h = lambda k, t=self.hostA: t[k][idx].numpy().astype(np.float64)
         gh = np.stack([h("gr"), h("gu")], -1)
         f = O.arz_rollout(h("r0"), h("u0"), gh, self.A["dx"], self.A["umax"], self.A["dt"], T)
         o = O.arz_rollout(h("r0"), h("u0"), gh, self.A["dx"], self.A["umax"], self.A["dt"], T,
                           g_rT=2.0 * (f["rT"] - h("tr")), g_uT=2.0 * (f["uT"] - h("tu")))
         rel = lambda x, y: float(np.abs(np.asarray(x, dtype=np.float64) - y).max() / (1e-300 + np.abs(y).max()))
-        sel = torch.tensor(idx)
         res = {"lanes": idx, "steps": T, "ckpt_every": self.K, "chunks": len(self.chunks),
                "arz": {"rT": rel(rT, o["rT"]), "uT": rel(uT, o["uT"]),
-                       "g_r0": rel(g_r0.cpu()[sel].numpy(), o["g_r0"]), "g_u0": rel(g_u0.cpu()[sel].numpy(), o["g_u0"])}}
+                       "g_r0": rel(cap["g_r0"].cpu().numpy(), o["g_r0"]), "g_u0": rel(cap["g_u0"].cpu().numpy(), o["g_u0"])}}
         # IDM: 32 sampled lanes (first, last, seeded)
         n, L = self.M["n"], self.hostM["head"].shape[0]
         lidx = sorted(set([0, L - 1] + [int(x) for x in rng.integers(0, L, 30)]))
@@ -587,6 +609,28 @@ class Batch:
         for k in ("arena", "devA", "devM", "hostA", "hostM"):
             setattr(self, k, None)
         self.torch.cuda.empty_cache()
+
+
+def dump_sample(n, bytes_per_item, budget):
+    """The sorted, seeded sample of items (lanes) of 0..n-1 whose outputs --dump-outputs writes: as many as fit the
+    budget, so the same arguments always select the same lanes."""
+    import numpy as np
+    k = min(n, max(1, budget // bytes_per_item))
+    return sorted(np.random.default_rng(SEED).choice(n, k, replace=False).tolist())
+
+
+def write_outputs(path, cap, losses, idm_lanes, lane_vehicles):
+    """--dump-outputs: the last timed pass's losses [arz, idm] and, for the sampled ARZ lanes and IDM lanes, the final
+    states and the gradients of the loss wrt the initial states, in the state dtype."""
+    import numpy as np
+    import torch
+    veh = torch.tensor([l * lane_vehicles + j for l in idm_lanes for j in range(lane_vehicles)], device=losses.device)
+    out = {"losses": losses}
+    out.update({"arz_" + k: cap[k] for k in ("rT", "yT", "uT", "g_r0", "g_u0")})
+    out.update({"idm_" + k: cap[k].index_select(0, veh) for k in ("pT", "vT", "g_p0", "g_v0")})
+    os.makedirs(path, exist_ok=True)
+    for name, t in out.items():
+        np.save(os.path.join(path, name + ".npy"), t.detach().cpu().numpy())
 
 
 def fp64_peak(dev, torch, lib):
@@ -641,8 +685,16 @@ def run_ours(a):
     bt = Batch(a, make_arz_inputs(a, rank, torch), make_idm_inputs(a, rank, torch), dev, dt_t, flags, torch)
     B, V = bt.B, bt.V
     clocks = Clocks(local) if rank == 0 else None
-    tm, losses, last_losses, (tw0, tw1) = bt.timed(a.steps, a.warmup, barrier)
+    cap = None
+    if a.dump_outputs and rank == 0:
+        arz_lanes = dump_sample(B, 5 * N * esz, DUMP_ARZ_BYTES)
+        idm_lanes = dump_sample(V // a.lane_vehicles, 4 * a.lane_vehicles * esz, DUMP_IDM_BYTES)
+        cap = bt.lane_capture(arz_lanes)
+    tm, losses, last_losses, (tw0, tw1) = bt.timed(a.steps, a.warmup, barrier, cap)
     clk = clocks.stop(tw0, tw1) if clocks else None
+    if cap is not None:
+        write_outputs(a.dump_outputs, cap, losses, idm_lanes, a.lane_vehicles)
+        del cap
     bits, ncol = flags.read()
     e2e_ms, h2d, d2h = (None, 0, 0)
     if not a.no_e2e:

@@ -13,7 +13,7 @@ with the signal-blended head deltas (_simulator.py:144-276), the cross-lane lead
 The routes ``create_random_route`` draws for spawned vehicles (road_network.py:604-646) are random INPUTS: they are
 recorded per vehicle, in spawn order per entry lane, and handed to the kernels as such.
 
-Fixture: tests/golden/itscp_hybrid_fp64.npz.
+Fixture: tests/golden/itscp_hybrid_<case>_fp64.npz (+ _hist0 / _hist1, see save_case).
 """
 import os
 import sys
@@ -200,9 +200,19 @@ def main():
     out.update(run_case("h", ItscpGrid(3, 1, 5.0, 5.0), T=T, frames_per_signal=30, seed=21))          # C4's geometry
     out.update(run_case("g", ItscpGrid(3, 1, 20.0, 5.0), T=T, frames_per_signal=24, seed=22))         # longer access lanes
     os.makedirs(OUT, exist_ok=True)
-    path = os.path.join(OUT, "itscp_hybrid_fp64.npz")
-    np.savez_compressed(path, **out)
-    print("wrote", path, os.path.getsize(path), "bytes")
+    for tag in ("h", "g"):
+        save_case(tag, {k[2:]: v for k, v in out.items() if k.startswith(tag + "_")})
+
+
+def save_case(tag, case):
+    """itscp_hybrid_<tag>_fp64.npz plus the state history in two halves along the frames, _hist0 / _hist1: every
+    stored file stays under 1 MB (tests/hyb_cases.fixture_case joins them)."""
+    hist = case.pop("hist")
+    half = (len(hist) + 1) // 2
+    for name, arrays in (("", case), ("_hist0", {"hist": hist[:half]}), ("_hist1", {"hist": hist[half:]})):
+        path = os.path.join(OUT, "itscp_hybrid_%s%s_fp64.npz" % (tag, name))
+        np.savez_compressed(path, **arrays)
+        print("wrote", path, os.path.getsize(path), "bytes")
 
 
 if __name__ == "__main__":

@@ -3,9 +3,10 @@
 run on top of the drop-in ``road/ model/ dmath/`` packages and must reproduce the curves frozen from the same
 drivers on the reference's own lanes (tests/golden/drivers_fp32.npz, oracle/gen_golden_drivers.py).
 
-The driver files live in the git-ignored reference install ``baseline/_ref`` (baseline/install_ref.py), which ships
-to the GPU box with the snapshot; the tests skip cleanly when it is absent.  One subprocess per problem: the
-drivers import ``road.*`` by name, and this pytest process may already hold other modules under those names.
+The driver files live in the git-ignored reference install ``baseline/_ref``, which baseline/install_ref.py copies
+from the checkout of the reference named by $DHTS_REFERENCE; the tests skip when it is absent.  One subprocess per
+problem: the drivers import ``road.*`` by name, and this pytest process may already hold other modules under those
+names.
 
 Two tiers, as everywhere in this suite (SURVEY 8c):
   * fp64 -- the drivers and the reference run in float64 (no-edit dtype rebinding, ``run_drivers.py --fp64``), the
@@ -30,7 +31,7 @@ from conftest import ROOT, golden, relerr
 def run_driver(problem, tmp_path, tier="fp32", defer=True, extra=()):
     ref = os.path.join(ROOT, "baseline", "_ref", "example", "inverse", problem + ".py")
     if not os.path.exists(ref):
-        pytest.skip("baseline/_ref is absent (python baseline/install_ref.py populates it where /root/reference exists)")
+        pytest.skip("baseline/_ref is absent (python baseline/install_ref.py populates it from $DHTS_REFERENCE)")
     g = golden("drivers_" + tier)
     out = str(tmp_path / (problem + ".npz"))
     env = dict(os.environ, DHTS_RUN_DIR=str(tmp_path))

@@ -9,8 +9,10 @@ F64 = torch.float64
 
 
 def fixture_case(tag):
-    g = golden("itscp_hybrid_fp64")
-    return {k[len(tag) + 1:]: g[k] for k in g.files if k.startswith(tag + "_")}
+    g = golden("itscp_hybrid_%s_fp64" % tag)
+    G = {k: g[k] for k in g.files}
+    G["hist"] = np.concatenate([golden("itscp_hybrid_%s_hist%d_fp64" % (tag, i))["hist"] for i in (0, 1)])
+    return G
 
 
 def t64(a, dev, grad=False):

@@ -4,8 +4,8 @@
     CUDA.  (2) The same end-to-end cases as tests/test_dropin_gpu.py, with the four kernel-backed calls swapped for
     the oracle-based stand-ins of tests/cpu_standin.py: everything ELSE -- marshalling between objects and vectors,
     boundary rules, spawn / absorb / hand-off bookkeeping, autograd wiring across lanes -- is the product code and is
-    checked against the live-reference fixtures.  (3) Where /root/reference is present (this container, not the GPU
-    box) the host-only rules are also compared with the live reference directly.
+    checked against the live-reference fixtures.  (3) Where $DHTS_REFERENCE names a checkout of the reference, the
+    host-only rules are also compared with the live reference directly.
 """
 import os
 import sys
@@ -95,7 +95,9 @@ def test_object_surface_host_logic():
 
 
 # ---------------------------------------------------------------------------------------------------------------
-# (3) host-only rules against the LIVE reference (skipped where /root/reference does not exist, e.g. the GPU box)
+# (3) host-only rules against the LIVE reference (skipped unless $DHTS_REFERENCE names a checkout of it)
+
+REF = os.environ.get("DHTS_REFERENCE", "")
 
 _PROBE = r'''
 import json, sys
@@ -150,7 +152,7 @@ print("PROBE" + json.dumps(out))
 '''
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/road"), reason="live reference not present on this box")
+@pytest.mark.skipif(not (REF and os.path.isdir(os.path.join(REF, "road"))), reason="$DHTS_REFERENCE: no checkout of the reference")
 def test_host_rules_match_live_reference():
     import json
     import subprocess
@@ -162,7 +164,7 @@ def test_host_rules_match_live_reference():
         assert r.returncode == 0, r.stderr[-2000:]
         return json.loads(r.stdout[r.stdout.index("PROBE") + 5:])
 
-    ref = run("", "/root/reference")
+    ref = run("", REF)
     ours = run("import dhts_b200.dropin as d; d.install()\n", root)
     assert ref["middle_insert"] == "AssertionError" and ref["too_close"] == "AssertionError"
     for k in ref:

@@ -1,6 +1,6 @@
 """Host side of the headless ITSCP env, trainer and log formats (no GPU): construction as run.py configures it,
-observation, schedules, MacroRoute draws against the live reference's, the running-mean sigmoid constants against a
-restatement of common/rms.py, and that stepping refuses to run without CUDA."""
+observation, schedules, MacroRoute draws against the reference's stored ones, the running-mean sigmoid constants
+against a restatement of common/rms.py, and that stepping refuses to run without CUDA."""
 import copy
 import os
 
@@ -8,9 +8,8 @@ import numpy as np
 import pytest
 import torch
 
+from hyb_cases import fixture_case
 from itscp_env_cases import c4_env, c4_fixture, c4_spawn_routes
-
-REF = os.environ.get("DHTS_REFERENCE", "/root/reference")
 
 
 def test_env_surface_matches_run_py_configuration():
@@ -100,38 +99,16 @@ def test_running_mean_constants_match_rms_restatement():
         assert np.abs(got[valid] - want[valid]).max() < 1e-9 * np.abs(want).max()
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="live reference not present")
 def test_macro_route_draws_follow_the_reference_rng_order():
-    """_make_macro_route consumes np.random exactly as ItscpRoadNetwork.create_random_macro_route does."""
-    import sys
-    sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle"))
-    from gen_golden_net import load_reference_simulator
-    saved = {k: v for k, v in sys.modules.items() if k.split(".")[0] in ("road", "model", "dmath", "example")}
-    for k in saved:
-        del sys.modules[k]
-    sys.path.insert(0, REF)
-    try:
-        ItscpRoadNetwork, _ = load_reference_simulator()
-        from road.lane.dmacro_lane import dMacroLane
-        from road.lane.dmicro_lane import dMicroLane
-        G = c4_fixture()
-        env = c4_env(G, "cpu")
-        net = ItscpRoadNetwork(60.0)
-        for info, k in zip(env.grid.lanes, env.kind):
-            net.add_lane(dMicroLane(len(net.lane), info.length, 60.0) if k else dMacroLane(len(net.lane), info.length, 60.0, 5.0))
-        for a, b in env.grid.links:
-            net.connect_lane(a, b)
-        env.num_timestep = 5
-        np.random.seed(11); env._make_macro_route()
-        np.random.seed(11)
-        ref = [net.create_random_macro_route() for _ in range(5)]
-        tab = np.array([[[r.get_prev_lane(l) for l in range(144)], [r.get_next_lane(l) for l in range(144)]] for r in ref])
-        assert (env.macro_route_schedule.numpy() == tab).all()
-    finally:
-        sys.path.remove(REF)
-        for k in [k for k in sys.modules if k.split(".")[0] in ("road", "model", "dmath", "example")]:
-            del sys.modules[k]
-        sys.modules.update(saved)
+    """_make_macro_route consumes np.random exactly as ItscpRoadNetwork.create_random_macro_route does: the hybrid
+    fixture's case h holds the reference's own draws on the config-4 grid, 120 frames after np.random.seed(21)
+    (oracle/gen_golden_hyb.py)."""
+    H = fixture_case("h")
+    env = c4_env(c4_fixture(), "cpu")
+    assert env.kind == H["kind"].tolist()
+    env.num_timestep = int(H["T"])
+    np.random.seed(21); env._make_macro_route()
+    assert (env.macro_route_schedule.numpy() == H["route"]).all()
 
 
 def test_trainer_log_formats(tmp_path):
