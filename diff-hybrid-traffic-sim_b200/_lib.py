@@ -24,7 +24,7 @@ SYMBOLS = [
     "dhts_version", "dhts_fp64_probe", "dhts_csr_expand", "dhts_idm_rollout_max_lane", "dhts_idm_rollout_max_ckpt_every", "dhts_hyb_aux_size",
 ] + [f"dhts_{op}_{suf}" for suf in ("f64", "f32") for op in (
     "arz_step_fwd", "arz_step_bwd", "arz_rollout_fwd", "arz_rollout_scratch_elems", "arz_rollout_ckpt_elems", "arz_rollout_bwd",
-    "idm_step_fwd", "idm_step_bwd", "idm_rollout_fwd", "idm_rollout_bwd",
+    "idm_step_fwd", "idm_step_bwd", "idm_step_bwd_params", "idm_rollout_fwd", "idm_rollout_bwd", "idm_rollout_bwd_params",
     "m2c_fwd", "m2c_bwd", "c2m_fwd", "c2m_bwd", "net_rollout_fwd", "net_rollout_bwd", "hyb_rollout_fwd", "hyb_rollout_bwd")]
 
 _lib = None

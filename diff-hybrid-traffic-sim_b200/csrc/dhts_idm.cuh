@@ -65,4 +65,42 @@ __device__ __forceinline__ void idm_jac(T v, const IdmPar<T>& k, T dp_raw, T dv_
     L11 = e.clip_acc ? T(0) : l11;
 }
 
+// Adjoint of the parameters (a_max, a_pref, v_target, s0, time_pref, length) of one vehicle, in factored form.  With
+// A = a_max, sd2 = s/dp^2, q = (v/v_t)^2 and acc the unclipped acceleration, nv = v + dt acc has
+//   d acc/d a_max  = acc/A + sd2 v dv sab2_inv        d acc/d a_pref = A sd2 v dv sab2_inv / a_pref
+//   d acc/d v_t    = 4 A q^2 v_t_inv                  d acc/d s0 = -2 A sd2      d acc/d time_pref = -2 A sd2 v
+//   d acc/d length = -A s^2/dp^3 = -(L10 / dt) / 2, for the own length and for the leader's.
+// Like idm_jac it uses e.s and the RAW deltas, so at collisions it follows the state Jacobian's convention; the
+// acceleration clip zeroes every term, a clipped s* (e.s = 0) every s term.  The per-vehicle constants of the rows are
+// left out, so that a rollout adjoint adds one product per step and parameter (idm_par_vjp) and applies them once at
+// the end (idm_par_grad).  The length row is not formed here: it is -cpv/2 (cpv = L10 gv, what the vehicle sends to
+// its leader) of the vehicle itself -- unless its gap is head_dp, which no length enters -- plus -cpv/2 of its follower.
+template <typename T> struct IdmParAdj { T acc, x, q2, sd2, sd2v, len; };
+
+template <typename T>
+__device__ __forceinline__ void idm_par_vjp(T v, const IdmPar<T>& k, T dp_raw, T dv_raw, const IdmEval<T>& e, T gv,
+                                            IdmParAdj<T>& a) {
+    if (e.clip_acc) return;
+    T idp = f_rcp(dp_raw);
+    T sd2 = e.s * idp * idp;
+    T q = (v * v) * (k.v_t_inv * k.v_t_inv);   // not idm_eval's q * q: sharing that product could unfuse its 1 - q*q
+    a.acc += gv * e.acc;
+    a.x += gv * (sd2 * (v * dv_raw));
+    a.q2 += gv * (q * q);
+    a.sd2 += gv * sd2;
+    a.sd2v += gv * (sd2 * v);
+}
+
+// g[6] = d loss / d params of the vehicle from its accumulated IdmParAdj (a_pref: the vehicle's raw parameter)
+template <typename T>
+__device__ __forceinline__ void idm_par_grad(const IdmParAdj<T>& a, const IdmPar<T>& k, T a_pref, T dt, T* g) {
+    const T A = k.a_max, xs = a.x * k.sab2_inv;
+    g[0] = dt * (a.acc / A + xs);
+    g[1] = dt * (A * xs / a_pref);
+    g[2] = dt * (T(4) * A * k.v_t_inv * a.q2);
+    g[3] = dt * (T(-2) * A * a.sd2);
+    g[4] = dt * (T(-2) * A * a.sd2v);
+    g[5] = a.len;
+}
+
 }  // namespace dhts

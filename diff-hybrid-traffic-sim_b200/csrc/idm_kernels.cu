@@ -53,18 +53,22 @@ idm_step_fwd_kernel(const T* __restrict__ p, const T* __restrict__ v, const T* _
     }
 }
 
-template <typename T>
+// PAR: also the adjoint of the vehicle parameters, g_params [6][V] (idm_par_vjp); a separate instantiation, so that the
+// state adjoint alone stays as it was.
+template <typename T, bool PAR>
 __global__ void __launch_bounds__(IDM_BLOCK)
 idm_step_bwd_kernel(const T* __restrict__ p, const T* __restrict__ v, const T* __restrict__ params,
                     const int* __restrict__ lane_off, const int* __restrict__ veh_lane, const T* __restrict__ head,
                     T dt, int V, const T* __restrict__ g_np, const T* __restrict__ g_nv, T* __restrict__ g_p,
-                    T* __restrict__ g_v, T* __restrict__ g_head, int* __restrict__ flags) {
+                    T* __restrict__ g_v, T* __restrict__ g_head, int* __restrict__ flags, T* __restrict__ g_params) {
     __shared__ T s_cp[IDM_BLOCK], s_cv[IDM_BLOCK];
     const int i = blockIdx.x * IDM_BLOCK + threadIdx.x;
     const bool valid = i < V;
     const T inv_dt = T(1) / dt;
-    // evaluate vehicle j against its leader; returns adjoint pieces
-    auto eval = [&](int j, T& E10, T& E11, T& L10, T& L11, bool& is_head, int& l) {
+    IdmParAdj<T> pa = {T(0), T(0), T(0), T(0), T(0), T(0)};
+    IdmPar<T> pk;
+    // evaluate vehicle j against its leader; returns adjoint pieces (and, for the thread's own vehicle, its parameter ones)
+    auto eval = [&](int j, T& E10, T& E11, T& L10, T& L11, bool& is_head, int& l, bool own) {
         T pj = p[j], vj = v[j];
         IdmPar<T> k = load_par(params, (size_t)V, (size_t)j);
         l = veh_lane[j];
@@ -74,14 +78,16 @@ idm_step_bwd_kernel(const T* __restrict__ p, const T* __restrict__ v, const T* _
         else { dp = t_abs(p[j + 1] - pj) - (params[5 * (size_t)V + j + 1] + k.len) * T(0.5); dv = vj - v[j + 1]; }
         IdmEval<T> e = idm_eval(vj, k, dp, dv, inv_dt);
         idm_jac(vj, k, dp, dv, e, dt, E10, E11, L10, L11);
+        if constexpr (PAR) if (own) { pk = k; idm_par_vjp(vj, k, dp, dv, e, g_nv[j], pa); }
     };
     T gp = T(0), gv = T(0), cp = T(0), cv = T(0);
     bool is_head = false; int l = 0;
     T E10 = 0, E11 = 0, L10, L11;
     if (valid) {
-        eval(i, E10, E11, L10, L11, is_head, l);
+        eval(i, E10, E11, L10, L11, is_head, l, true);
         gp = g_np[i]; gv = g_nv[i];
         cp = L10 * gv; cv = L11 * gv;     // L^T g: what this vehicle sends to its leader
+        if constexpr (PAR) if (!is_head) pa.len = T(-0.5) * cp;
     }
     s_cp[threadIdx.x] = cp; s_cv[threadIdx.x] = cv;
     __syncthreads();
@@ -90,12 +96,15 @@ idm_step_bwd_kernel(const T* __restrict__ p, const T* __restrict__ v, const T* _
     T ov = dt * gp + E11 * gv;
     const bool is_tail = (i == lane_off[l]);
     if (!is_tail) {                       // contribution of the follower i-1
-        if (threadIdx.x > 0) { op += s_cp[threadIdx.x - 1]; ov += s_cv[threadIdx.x - 1]; }
-        else {
+        if (threadIdx.x > 0) {
+            op += s_cp[threadIdx.x - 1]; ov += s_cv[threadIdx.x - 1];
+            if constexpr (PAR) pa.len += T(-0.5) * s_cp[threadIdx.x - 1];
+        } else {
             T e10, e11, l10, l11; bool h; int ll;
-            eval(i - 1, e10, e11, l10, l11, h, ll);
+            eval(i - 1, e10, e11, l10, l11, h, ll, false);
             T gvf = g_nv[i - 1];
             op += l10 * gvf; ov += l11 * gvf;
+            if constexpr (PAR) pa.len += (T(-0.5) * l10) * gvf;     // not l10 * gvf: that product must stay fused into op
         }
     }
     if (is_head) {                        // ghost leader = (p_head + dp, v_head - dv), dmicro_lane.py:144-151
@@ -103,7 +112,14 @@ idm_step_bwd_kernel(const T* __restrict__ p, const T* __restrict__ v, const T* _
         if (g_head) { g_head[2 * l] = cp; g_head[2 * l + 1] = -cv; }
     }
     g_p[i] = op; g_v[i] = ov;
-    if (t_isnan(op) || t_isnan(ov)) atomicOr(flags, FLAG_NAN_GRAD);
+    bool nan = t_isnan(op) || t_isnan(ov);
+    if constexpr (PAR) {
+        T g[6];
+        idm_par_grad(pa, pk, params[(size_t)V + i], dt, g);
+#pragma unroll
+        for (int r = 0; r < 6; r++) { g_params[(size_t)r * V + i] = g[r]; nan |= t_isnan(g[r]); }
+    }
+    if (nan) atomicOr(flags, FLAG_NAN_GRAD);
 }
 
 // lanes with no vehicle get a zero head gradient
@@ -225,13 +241,15 @@ idm_rollout_fwd_kernel(const T* __restrict__ p0, const T* __restrict__ v0, const
 }
 
 // EXT = false: no per-step head deltas, no per-step adjoint injection (head_t, g_head_t, g_hist are null).
-template <typename T, int VPT, bool EXT>
+// PAR = true: also the adjoint of the vehicle parameters, g_params [6][V]: each thread keeps six accumulators per vehicle
+// in registers over all segments (idm_par_vjp) and writes them once, after the last step.
+template <typename T, int VPT, bool EXT, bool PAR>
 __global__ void __launch_bounds__(IDM_ROLL_BLOCK)
 idm_rollout_bwd_kernel(const T* __restrict__ ckpt, const T* __restrict__ params, const int* __restrict__ lane_off,
                        const T* __restrict__ head, const T* __restrict__ head_t_, T dt, int V, int L, int steps, int K,
                        const T* __restrict__ g_pT, const T* __restrict__ g_vT, const T* __restrict__ g_hist_,
                        T* __restrict__ g_p0, T* __restrict__ g_v0, T* __restrict__ g_head, T* __restrict__ g_head_t_,
-                       int* __restrict__ flags) {
+                       int* __restrict__ flags, T* __restrict__ g_params) {
     const T* __restrict__ head_t = EXT ? head_t_ : nullptr;
     const T* __restrict__ g_hist = EXT ? g_hist_ : nullptr;
     T* __restrict__ g_head_t = EXT ? g_head_t_ : nullptr;
@@ -252,10 +270,12 @@ idm_rollout_bwd_kernel(const T* __restrict__ ckpt, const T* __restrict__ params,
         T hdp = head_t ? T(0) : head[2 * l], hdv = head_t ? T(0) : head[2 * l + 1];
         WarpLane<T, VPT> w;
         T gp[VPT], gv[VPT], ghp = T(0), ghv = T(0);
+        IdmParAdj<T> pa[VPT];
 #pragma unroll
         for (int m = 0; m < VPT; m++) {
             int e = m * 32 + (int)lane;
             gp[m] = (e < n) ? g_pT[o + e] : T(0); gv[m] = (e < n) ? g_vT[o + e] : T(0);
+            if constexpr (PAR) pa[m] = {T(0), T(0), T(0), T(0), T(0), T(0)};
         }
         for (int seg = S - 1; seg >= 0; seg--) {
             const int t0 = seg * K, ks = min(K, steps - t0);
@@ -283,6 +303,11 @@ idm_rollout_bwd_kernel(const T* __restrict__ ckpt, const T* __restrict__ params,
                     nv_[m] = dt * gp[m] + E11 * gv[m];
                     cpv[m] = L10 * gv[m]; cvv[m] = L11 * gv[m];
                     if (w.head[m]) { np_[m] += cpv[m]; nv_[m] += cvv[m]; ghp += cpv[m]; ghv -= cvv[m]; }
+                    if constexpr (PAR)
+                        if (w.valid[m]) {
+                            idm_par_vjp(w.v[m], w.k[m], dp[m], dv[m], e, gv[m], pa[m]);
+                            if (!w.head[m]) pa[m].len += T(-0.5) * cpv[m];
+                        }
                 }
                 // follower (e-1) -> me: within a slot from lane-1, across slots from lane 31 of slot m-1
 #pragma unroll
@@ -292,6 +317,7 @@ idm_rollout_bwd_kernel(const T* __restrict__ ckpt, const T* __restrict__ params,
                     const T sv_ = (lane == 31) ? (m > 0 ? cvv[m > 0 ? m - 1 : 0] : T(0)) : cvv[m];
                     const T fp = __shfl_sync(0xffffffffu, sp_, (lane + 31) & 31), fv = __shfl_sync(0xffffffffu, sv_, (lane + 31) & 31);
                     if (w.valid[m]) { gp[m] = np_[m] + fp; gv[m] = nv_[m] + fv; }
+                    if constexpr (PAR) pa[m].len += T(-0.5) * fp;      // the follower's gap holds this vehicle's length
                 }
                 if (g_head_t) {       // per-step head deltas: this step's adjoint leaves, the accumulator restarts
                     bool own = false;
@@ -315,6 +341,17 @@ idm_rollout_bwd_kernel(const T* __restrict__ ckpt, const T* __restrict__ params,
 #pragma unroll
         for (int m = 0; m < VPT; m++)
             if (w.valid[m]) { g_p0[o + m * 32 + lane] = gp[m]; g_v0[o + m * 32 + lane] = gv[m]; }
+        if constexpr (PAR) {
+#pragma unroll
+            for (int m = 0; m < VPT; m++)
+                if (w.valid[m]) {
+                    const size_t i = (size_t)o + m * 32 + lane;
+                    T g[6];
+                    idm_par_grad(pa[m], w.k[m], params[(size_t)V + i], dt, g);
+#pragma unroll
+                    for (int r = 0; r < 6; r++) { g_params[(size_t)r * V + i] = g[r]; bad |= t_isnan(g[r]); }
+                }
+        }
         if (g_head) {
             // exactly one thread of the warp owns the head vehicle
             bool own = false;
@@ -352,18 +389,23 @@ static int idm_step_fwd(const T* p, const T* v, const T* params, const int* lane
     return last_status_idm();
 }
 
+// g_params NULL: the state adjoint only (dhts_idm_step_bwd_*)
 template <typename T>
 static int idm_step_bwd(const T* p, const T* v, const T* params, const int* lane_off, const int* veh_lane,
                         const T* head, T dt, int V, int L, const T* g_np, const T* g_nv, T* g_p, T* g_v, T* g_head,
-                        int* flags, cudaStream_t st) {
+                        T* g_params, int* flags, cudaStream_t st) {
     if (!p || !v || !params || !lane_off || !veh_lane || !head || !g_np || !g_nv || !g_p || !g_v || !flags || V < 0 ||
         L < 0)
         return DHTS_ERR_INVALID;
     if (g_head && L > 0) idm_zero_empty_head_kernel<T><<<(L + 255) / 256, 256, 0, st>>>(lane_off, L, g_head);
     if (V == 0) return last_status_idm();
-    idm_step_bwd_kernel<T><<<(V + IDM_BLOCK - 1) / IDM_BLOCK, IDM_BLOCK, 0, st>>>(p, v, params, lane_off, veh_lane, head,
-                                                                                  dt, V, g_np, g_nv, g_p, g_v, g_head,
-                                                                                  flags);
+    const int grid = (V + IDM_BLOCK - 1) / IDM_BLOCK;
+    if (g_params)
+        idm_step_bwd_kernel<T, true><<<grid, IDM_BLOCK, 0, st>>>(p, v, params, lane_off, veh_lane, head, dt, V, g_np, g_nv,
+                                                                 g_p, g_v, g_head, flags, g_params);
+    else
+        idm_step_bwd_kernel<T, false><<<grid, IDM_BLOCK, 0, st>>>(p, v, params, lane_off, veh_lane, head, dt, V, g_np, g_nv,
+                                                                  g_p, g_v, g_head, flags, nullptr);
     return last_status_idm();
 }
 
@@ -391,10 +433,11 @@ static int idm_rollout_fwd(const T* p0, const T* v0, const T* params, const int*
     return last_status_idm();
 }
 
+// g_params NULL: the state adjoint only (dhts_idm_rollout_bwd_*)
 template <typename T>
 static int idm_rollout_bwd(const T* ckpt, const T* params, const int* lane_off, const T* head, const T* head_t, T dt, int V,
                            int L, int max_lane, int steps, int K, const T* g_pT, const T* g_vT, const T* g_hist, T* g_p0,
-                           T* g_v0, T* g_head, T* g_head_t, int* flags, cudaStream_t st) {
+                           T* g_v0, T* g_head, T* g_head_t, T* g_params, int* flags, cudaStream_t st) {
     if (!ckpt || !params || !lane_off || (!head && !head_t) || !g_pT || !g_vT || !g_p0 || !g_v0 || !flags || V < 0 || L < 0 ||
         steps < 0 || max_lane < 0 || K < 1)
         return DHTS_ERR_INVALID;
@@ -402,10 +445,13 @@ static int idm_rollout_bwd(const T* ckpt, const T* params, const int* lane_off, 
     if (K > IDM_KMAX) return DHTS_ERR_UNSUPPORTED;
     if (L == 0) return DHTS_OK;
     int grid = idm_grid(L);
-#define CALL(VPT) { if (head_t || g_hist || g_head_t) idm_rollout_bwd_kernel<T, VPT, true><<<grid, IDM_ROLL_BLOCK, 0, st>>>(ckpt, params, lane_off, head, head_t, dt, V, L, steps, K, g_pT, g_vT, g_hist, g_p0, g_v0, head_t ? nullptr : g_head, g_head_t, flags); \
-                    else idm_rollout_bwd_kernel<T, VPT, false><<<grid, IDM_ROLL_BLOCK, 0, st>>>(ckpt, params, lane_off, head, nullptr, dt, V, L, steps, K, g_pT, g_vT, nullptr, g_p0, g_v0, g_head, nullptr, flags); }
+    const bool ext = head_t || g_hist || g_head_t;
+#define LAUNCH(VPT, EXT, PAR) idm_rollout_bwd_kernel<T, VPT, EXT, PAR><<<grid, IDM_ROLL_BLOCK, 0, st>>>(ckpt, params, lane_off, head, EXT ? head_t : nullptr, dt, V, L, steps, K, g_pT, g_vT, EXT ? g_hist : nullptr, g_p0, g_v0, (EXT && head_t) ? nullptr : g_head, EXT ? g_head_t : nullptr, flags, g_params);
+#define CALL(VPT) { if (g_params) { if (ext) LAUNCH(VPT, true, true) else LAUNCH(VPT, false, true) } \
+                    else { if (ext) LAUNCH(VPT, true, false) else LAUNCH(VPT, false, false) } }
     DHTS_VPT_DISPATCH(max_lane, CALL)
 #undef CALL
+#undef LAUNCH
     return last_status_idm();
 }
 
@@ -422,7 +468,15 @@ static int idm_rollout_bwd(const T* ckpt, const T* params, const int* lane_off, 
                                             const int* veh_lane, const T* head, T dt, int V, int L, const T* g_np,     \
                                             const T* g_nv, T* g_p, T* g_v, T* g_head, int* flags, void* stream) {      \
         return dhts::idm_step_bwd<T>(p, v, params, lane_off, veh_lane, head, dt, V, L, g_np, g_nv, g_p, g_v, g_head,   \
-                                     flags, (cudaStream_t)stream);                                                     \
+                                     nullptr, flags, (cudaStream_t)stream);                                            \
+    }                                                                                                                  \
+    DHTS_EXPORT int dhts_idm_step_bwd_params_##SUF(const T* p, const T* v, const T* params, const int* lane_off,       \
+                                                   const int* veh_lane, const T* head, T dt, int V, int L,             \
+                                                   const T* g_np, const T* g_nv, T* g_p, T* g_v, T* g_head,            \
+                                                   T* g_params, int* flags, void* stream) {                            \
+        if (!g_params) return DHTS_ERR_INVALID;                                                                        \
+        return dhts::idm_step_bwd<T>(p, v, params, lane_off, veh_lane, head, dt, V, L, g_np, g_nv, g_p, g_v, g_head,   \
+                                     g_params, flags, (cudaStream_t)stream);                                           \
     }                                                                                                                  \
     DHTS_EXPORT int dhts_idm_rollout_fwd_##SUF(const T* p0, const T* v0, const T* params, const int* lane_off,         \
                                                const T* head, const T* head_t, T dt, int V, int L, int max_lane,       \
@@ -436,7 +490,17 @@ static int idm_rollout_bwd(const T* ckpt, const T* params, const int* lane_off, 
                                                int ckpt_every, const T* g_pT, const T* g_vT, const T* g_hist,          \
                                                T* g_p0, T* g_v0, T* g_head, T* g_head_t, int* flags, void* stream) {   \
         return dhts::idm_rollout_bwd<T>(ckpt, params, lane_off, head, head_t, dt, V, L, max_lane, steps, ckpt_every,   \
-                                        g_pT, g_vT, g_hist, g_p0, g_v0, g_head, g_head_t, flags,                       \
+                                        g_pT, g_vT, g_hist, g_p0, g_v0, g_head, g_head_t, nullptr, flags,              \
+                                        (cudaStream_t)stream);                                                         \
+    }                                                                                                                  \
+    DHTS_EXPORT int dhts_idm_rollout_bwd_params_##SUF(const T* ckpt, const T* params, const int* lane_off,             \
+                                                      const T* head, const T* head_t, T dt, int V, int L,              \
+                                                      int max_lane, int steps, int ckpt_every, const T* g_pT,          \
+                                                      const T* g_vT, const T* g_hist, T* g_p0, T* g_v0, T* g_head,     \
+                                                      T* g_head_t, T* g_params, int* flags, void* stream) {            \
+        if (!g_params) return DHTS_ERR_INVALID;                                                                        \
+        return dhts::idm_rollout_bwd<T>(ckpt, params, lane_off, head, head_t, dt, V, L, max_lane, steps, ckpt_every,   \
+                                        g_pT, g_vT, g_hist, g_p0, g_v0, g_head, g_head_t, g_params, flags,             \
                                         (cudaStream_t)stream);                                                         \
     }
 

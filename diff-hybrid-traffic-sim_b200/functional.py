@@ -125,7 +125,9 @@ def arz_rollout_plan(B, N, steps, dtype, device, mem_fraction=0.6, min_lanes=296
 
 def idm_step(p, v, params, lane_off, head, dt, flags, veh_lane=None, want_flags=False):
     """One IDM step of all lanes: the batched dMicroForwardLayer.apply (dmicro_lane.py:75).
-    Returns (np, nv)[V] (+ per-vehicle clip / collision bits)."""
+    Returns (np, nv)[V] (+ per-vehicle clip / collision bits).  params [6, V] (a_max, a_pref, v_target, s0, time_pref,
+    length) is differentiable; for one parameter set shared by many vehicles pass a [6, 1] leaf ``.expand(6, V)``:
+    autograd sums the per-vehicle gradients into it."""
     if veh_lane is None:
         veh_lane = csr_expand(lane_off, p.numel())
     return IdmStepFn.apply(p, v, head, params, lane_off, veh_lane, dt, flags.t, want_flags)
@@ -136,7 +138,10 @@ def idm_rollout(p0, v0, params, lane_off, head, dt, steps, ckpt_every=32, flags=
     (head_position_delta, head_speed_delta): the loop of example/inverse/_inverse.py:91-99 for
     example/inverse/micro.py, batched.  head [L, 2], or [steps, L, 2] for one pair per step (needs no special
     checkpointing).  Returns (pT, vT) [V]; with return_history=True (ckpt_every = 1) also (p_hist, v_hist) [steps, V],
-    the state BEFORE every step, differentiable (a loss may read the lanes at every step)."""
+    the state BEFORE every step, differentiable (a loss may read the lanes at every step).  params [6, V] is
+    differentiable (calibration of the driver model against trajectories); a parameter set shared by many vehicles is a
+    [6, 1] leaf ``.expand(6, V)`` (or, one set per lane, a [6, L] leaf indexed by each vehicle's lane), and autograd
+    sums the per-vehicle gradients into it."""
     flags = flags or _lib.Flags(p0.device)
     if max_lane is None:
         max_lane = int((lane_off[1:] - lane_off[:-1]).max().item()) if lane_off.numel() > 1 else 0

@@ -219,7 +219,7 @@ def csr_expand(lane_off: torch.Tensor, V: int) -> torch.Tensor:
 
 
 class IdmStepFn(torch.autograd.Function):
-    """(p, v)[V], head[L,2] -> (np, nv)[V]; params [6,V], CSR lane_off[L+1]."""
+    """(p, v)[V], head[L,2] -> (np, nv)[V]; params [6,V] (differentiable), CSR lane_off[L+1]."""
 
     @staticmethod
     def forward(ctx, p, v, head, params, lane_off, veh_lane, dt, flags, want_flags):
@@ -251,11 +251,17 @@ class IdmStepFn(torch.autograd.Function):
         g_np, g_nv = z(g_np), z(g_nv)
         g_p = torch.empty_like(p); g_v = torch.empty_like(p)
         g_head = torch.zeros_like(head)
+        args = (ptr(p), ptr(v), ptr(params), ptr(lane_off), ptr(veh_lane), ptr(head), creal(p.dtype, ctx.dt), V, L,
+                ptr(g_np), ptr(g_nv), ptr(g_p), ptr(g_v), ptr(g_head))
+        g_params = None
         with torch.cuda.device(dev):
-            check(_fn("idm_step_bwd", p.dtype)(ptr(p), ptr(v), ptr(params), ptr(lane_off), ptr(veh_lane), ptr(head),
-                                               creal(p.dtype, ctx.dt), V, L, ptr(g_np), ptr(g_nv), ptr(g_p), ptr(g_v),
-                                               ptr(g_head), ptr(flags), stream_ptr(dev)), "dhts_idm_step_bwd")
-        return g_p, g_v, g_head, None, None, None, None, None, None
+            if ctx.needs_input_grad[3]:
+                g_params = torch.empty_like(params)
+                check(_fn("idm_step_bwd_params", p.dtype)(*args, ptr(g_params), ptr(flags), stream_ptr(dev)),
+                      "dhts_idm_step_bwd_params")
+            else:
+                check(_fn("idm_step_bwd", p.dtype)(*args, ptr(flags), stream_ptr(dev)), "dhts_idm_step_bwd")
+        return g_p, g_v, g_head, g_params, None, None, None, None, None
 
 
 class IdmRolloutFn(torch.autograd.Function):
@@ -263,7 +269,8 @@ class IdmRolloutFn(torch.autograd.Function):
 
     head [L,2]: one (head_position_delta, head_speed_delta) pair per lane for the whole rollout; head [steps,L,2]: one
     pair PER STEP (inside a network setup_micro_boundary rewrites them every step, road_network.py:429-580).
-    want_hist (ckpt_every = 1): a third output hist [steps,2,V], (p, v) BEFORE every step, differentiable."""
+    want_hist (ckpt_every = 1): a third output hist [steps,2,V], (p, v) BEFORE every step, differentiable.
+    params [6,V] is differentiable too: its adjoint accumulates over every step in the adjoint kernel."""
 
     @staticmethod
     def forward(ctx, p0, v0, head, params, lane_off, max_lane, dt, steps, ckpt_every, flags, want_hist=False):
@@ -278,7 +285,7 @@ class IdmRolloutFn(torch.autograd.Function):
             assert head.shape == (steps, L, 2), "per-step head deltas are [steps, L, 2]"
         if want_hist and K != 1:
             raise ValueError("the state history needs ckpt_every = 1 (every state stored)")
-        need_grad = any(ctx.needs_input_grad[i] for i in (0, 1, 2))
+        need_grad = any(ctx.needs_input_grad[i] for i in (0, 1, 2, 3))
         S = (steps + K - 1) // K
         ckpt = torch.empty((S, 2, max(V, 1)), dtype=p0.dtype, device=dev) if (need_grad or want_hist) else None
         pT = torch.empty_like(p0); vT = torch.empty_like(p0)
@@ -306,13 +313,18 @@ class IdmRolloutFn(torch.autograd.Function):
         g_hist = _c(g_hist)
         g_p0 = torch.empty((V,), dtype=dtype, device=dev); g_v0 = torch.empty_like(g_p0)
         g_head = torch.zeros_like(head)
+        args = (ptr(ckpt), ptr(params), ptr(lane_off), ptr(None if tv else head), ptr(head if tv else None),
+                creal(dtype, dt_), V, L, max_lane, steps, K, ptr(g_pT), ptr(g_vT), ptr(g_hist), ptr(g_p0), ptr(g_v0),
+                ptr(None if tv else g_head), ptr(g_head if tv else None))
+        g_params = None
         with torch.cuda.device(dev):
-            check(_fn("idm_rollout_bwd", dtype)(ptr(ckpt), ptr(params), ptr(lane_off), ptr(None if tv else head),
-                                                ptr(head if tv else None), creal(dtype, dt_), V, L, max_lane, steps, K,
-                                                ptr(g_pT), ptr(g_vT), ptr(g_hist), ptr(g_p0), ptr(g_v0),
-                                                ptr(None if tv else g_head), ptr(g_head if tv else None), ptr(flags),
-                                                stream_ptr(dev)), "dhts_idm_rollout_bwd")
-        return g_p0, g_v0, g_head, None, None, None, None, None, None, None, None
+            if ctx.needs_input_grad[3]:
+                g_params = torch.empty_like(params)
+                check(_fn("idm_rollout_bwd_params", dtype)(*args, ptr(g_params), ptr(flags), stream_ptr(dev)),
+                      "dhts_idm_rollout_bwd_params")
+            else:
+                check(_fn("idm_rollout_bwd", dtype)(*args, ptr(flags), stream_ptr(dev)), "dhts_idm_rollout_bwd")
+        return g_p0, g_v0, g_head, g_params, None, None, None, None, None, None, None
 
 
 class MacroToMicroFn(torch.autograd.Function):

@@ -186,6 +186,21 @@ int dhts_idm_step_bwd_f32(const float* p, const float* v, const float* params, c
                           const int* veh_lane, const float* head, float dt, int V, int L, const float* g_np,
                           const float* g_nv, float* g_p, float* g_v, float* g_head, int* flags, void* stream);
 
+/* The same, plus the adjoint of the vehicle parameters: g_params [6][V], laid out like params, every entry written
+ * (not accumulated).  Like the state Jacobian it is taken with the raw gap and speed difference, so at a collision it
+ * follows the same convention; a clipped acceleration contributes nothing, a clipped s* no s-term.  The head vehicle's
+ * gap is head_dp, so its own length enters only through its follower's gap.  NULL g_params returns
+ * DHTS_ERR_INVALID; a NaN parameter adjoint sets DHTS_FLAG_NAN_GRAD.  g_p, g_v, g_head are those of
+ * dhts_idm_step_bwd_*, bit for bit. */
+int dhts_idm_step_bwd_params_f64(const double* p, const double* v, const double* params, const int* lane_off,
+                                 const int* veh_lane, const double* head, double dt, int V, int L, const double* g_np,
+                                 const double* g_nv, double* g_p, double* g_v, double* g_head, double* g_params,
+                                 int* flags, void* stream);
+int dhts_idm_step_bwd_params_f32(const float* p, const float* v, const float* params, const int* lane_off,
+                                 const int* veh_lane, const float* head, float dt, int V, int L, const float* g_np,
+                                 const float* g_nv, float* g_p, float* g_v, float* g_head, float* g_params, int* flags,
+                                 void* stream);
+
 /* ---------------------------------------------------------------- IDM, fused T-step rollout
  * One warp per lane, vehicles in registers, leaders by warp shuffle.  max_lane =
  * largest lane size (<= dhts_idm_rollout_max_lane()); ckpt [S][2][V];
@@ -211,6 +226,18 @@ int dhts_idm_rollout_bwd_f32(const float* ckpt, const float* params, const int* 
                              const float* head_t, float dt, int V, int L, int max_lane, int steps, int ckpt_every,
                              const float* g_pT, const float* g_vT, const float* g_hist, float* g_p0, float* g_v0,
                              float* g_head, float* g_head_t, int* flags, void* stream);
+/* The same, plus the adjoint of the vehicle parameters over the whole rollout: g_params [6][V], with the convention,
+ * validation and flags of dhts_idm_step_bwd_params_*.  Per-step head deltas and g_hist are taken as above.  g_p0, g_v0,
+ * g_head, g_head_t are those of dhts_idm_rollout_bwd_*, bit for bit. */
+int dhts_idm_rollout_bwd_params_f64(const double* ckpt, const double* params, const int* lane_off, const double* head,
+                                    const double* head_t, double dt, int V, int L, int max_lane, int steps,
+                                    int ckpt_every, const double* g_pT, const double* g_vT, const double* g_hist,
+                                    double* g_p0, double* g_v0, double* g_head, double* g_head_t, double* g_params,
+                                    int* flags, void* stream);
+int dhts_idm_rollout_bwd_params_f32(const float* ckpt, const float* params, const int* lane_off, const float* head,
+                                    const float* head_t, float dt, int V, int L, int max_lane, int steps, int ckpt_every,
+                                    const float* g_pT, const float* g_vT, const float* g_hist, float* g_p0, float* g_v0,
+                                    float* g_head, float* g_head_t, float* g_params, int* flags, void* stream);
 
 /* ---------------------------------------------------------------- macro <-> micro exchange (per junction)
  * macro -> micro, road/network/conversion.py:15-73 (with MacroLane.add_flux_capacitor,
