@@ -155,18 +155,6 @@ arz_step_bwd_kernel(const T* __restrict__ r_pad, const T* __restrict__ y_pad, co
 
 // ------------------------------------------------------------------ host-side launch planning
 
-template <typename K> static int ensure_smem(K kernel, size_t bytes) {
-    if (bytes > 48 * 1024) {
-        if (cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes) != cudaSuccess) {
-            cudaGetLastError();
-            return DHTS_ERR_CUDA;
-        }
-    }
-    return DHTS_OK;
-}
-
-static int last_status() { return cudaGetLastError() == cudaSuccess ? DHTS_OK : DHTS_ERR_CUDA; }
-
 template <typename T>
 static int arz_step_fwd(const T* r_pad, const T* y_pad, const T* u_pad, const T* ueq_pad, const T* dx, const T* umax,
                         T dt, int B, int N, T* nr, T* ny, T* nu, int* case_out, int* flags, cudaStream_t st) {
@@ -177,7 +165,7 @@ static int arz_step_fwd(const T* r_pad, const T* y_pad, const T* u_pad, const T*
     size_t sm = smem_bytes<T, false>(STEP_TILE + 2, STEP_TILE + 1);
     arz_step_fwd_kernel<T><<<B * ntile, STEP_TILE, sm, st>>>(r_pad, y_pad, u_pad, ueq_pad, dx, umax, dt, B, N, ntile, nr,
                                                               ny, nu, case_out, flags);
-    return last_status();
+    return launch_status();
 }
 
 template <typename T>
@@ -191,11 +179,11 @@ static int arz_step_bwd(const T* r_pad, const T* y_pad, const T* u_pad, const T*
     int ntile = (N + STEP_TILE - 1) / STEP_TILE;
     if ((long long)B * ntile > 2147483647LL) return DHTS_ERR_UNSUPPORTED;
     size_t sm = smem_bytes<T, true>(STEP_TILE + 2, STEP_TILE + 1);
-    int rc = ensure_smem(arz_step_bwd_kernel<T>, sm);
+    int rc = set_smem(arz_step_bwd_kernel<T>, sm);
     if (rc) return rc;
     arz_step_bwd_kernel<T><<<B * ntile, STEP_TILE, sm, st>>>(r_pad, y_pad, u_pad, ueq_pad, dx, umax, dt, B, N, ntile, nr,
                                                               ny, g_nr, g_ny, g_nu, g_r_pad, g_y_pad, flags);
-    return last_status();
+    return launch_status();
 }
 
 }  // namespace dhts

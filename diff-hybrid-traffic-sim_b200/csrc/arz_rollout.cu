@@ -20,7 +20,7 @@
 // and the autograd chain through them (example/inverse/_inverse.py:91-99,227;
 // road/lane/dmacro_lane.py:68-132,234-310).
 #include <cstdint>
-#include <cstdlib>
+#include <type_traits>
 #define DHTS_CONSTANT_BANK_LITERALS      // see dhts_arz.cuh (KC)
 #include "dhts_arz_lean.cuh"
 #include "dhts_api.h"
@@ -115,7 +115,7 @@ __device__ __forceinline__ void from_right(const T* mine, T* out, T* box, int wa
     }
 }
 
-// Chunk loads / stores.  C > 1 is only planned when every row start is 16-byte aligned (plan_reg), so the
+// Chunk loads / stores.  C > 1 is only planned when every row start is 16-byte aligned (fwd_plan, bwd_plan), so the
 // vector forms are unconditional.
 template <typename T, int C> struct Chunk;
 template <typename T> struct Chunk<T, 1> {
@@ -824,55 +824,50 @@ __global__ void __launch_bounds__(1024 / (C < 4 ? C : 4), MB) arz_rollout_bwd_re
 }
 
 // ------------------------------------------------------------------ host-side planning and launch
+//
+// fwd_plan / bwd_plan alone decide what a call runs: from the shape and the call's options they fix every template argument
+// and the launch shape.  fwd_kernel / bwd_kernel map a plan to its instantiation; their lists are every instantiation this
+// file compiles.
 
-struct RegPlan { int C, lpc, threads, grid, ring_ns, mode; size_t smem; };
+// Measured on B200 (profiles/r1e sweep, fp64, 8192 lanes x 1024 cells): both kernels are fastest with 4 cells per
+// thread capped at 128 registers (2 CTAs of 256 threads per SM) -- forward 57 ms vs 69-89 ms for the other
+// shapes, adjoint 97 ms (every state stored) / 149 ms (K = 32) vs 106-226 ms.
+constexpr int CELLS = 4;                      // cells per thread where the lane allows (2 or 8: 1530 / 996 ms per pass against 938, r2)
+constexpr int RING_NS = 4;                    // adjoint ring stages (3 or 6: 940 / 939 ms per pass against 938, r2)
+constexpr int NSF = 4;                        // staging stages of the forward kernel
+// Staging ring / state ring per CTA: keeps two CTAs of the 128-register shape on an SM (227 KB usable, 1 KB reserved per CTA).
+constexpr size_t RING_BUDGET = 112 * 1024;
+// Up to this much shared memory the C = 4 staged forward kernels run at 80 registers, three CTAs per SM (MB = 3): 384 vs
+// 393 ms per pass (r2c A/B), 391 vs 405 ms with the stored outcomes (r2u A/B).
+constexpr size_t MB3_BUDGET = 74 * 1024;
+
+// Template arguments of a launch.  MB is the register budget in units of "CTAs of 1024/min(C,4) threads per SM": 2 -> 128
+// registers (measured best for every C > 1, profiles/r1e sweep), 3 -> 80, 1 -> 255.
+struct FwdKey { int C, MB, NS; bool TV, XR, UNI; };
+struct BwdKey { int C, MB, MODE; bool EXT, XR, UNI; };
+static bool operator==(const FwdKey& a, const FwdKey& b) {
+    return a.C == b.C && a.MB == b.MB && a.NS == b.NS && a.TV == b.TV && a.XR == b.XR && a.UNI == b.UNI;
+}
+static bool operator==(const BwdKey& a, const BwdKey& b) {
+    return a.C == b.C && a.MB == b.MB && a.MODE == b.MODE && a.EXT == b.EXT && a.XR == b.XR && a.UNI == b.UNI;
+}
+template <typename Key> struct Plan {
+    Key k;
+    int lpc, threads, groups;     // lanes per CTA, threads per CTA, lane groups (CTAs of a non-persistent launch)
+    int ring_ns;                  // stages of the adjoint's state ring (MODE 0), else 0
+    size_t smem;
+    RollK rk;
+};
 
 static int round32(int x) { return (x + 31) / 32 * 32; }
 // vector chunk loads need 16-byte aligned bases (row offsets are multiples of C elements by construction)
 static bool al16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
-static int sm_count_r() {
-    static int n = 0;
-    if (!n) {
-        int dev = 0; cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
-        if (n <= 0) n = 148;
-    }
-    return n;
-}
-
-// Measured on B200 (profiles/r1e sweep, fp64, 8192 lanes x 1024 cells): both kernels are fastest with 4 cells per
-// thread capped at 128 registers (2 CTAs of 256 threads per SM) -- forward 57 ms vs 69-89 ms for the other
-// shapes, adjoint 97 ms (every state stored) / 149 ms (K = 32) vs 106-226 ms.
-// Tuning knobs (environment), read ONCE per process: cells per thread, adjoint ring stages, forward staging.
-struct Knobs { int c_fwd, c_bwd, ring, stage, mb_fwd, xrow, mb_xfwd, uni; };
-static const Knobs& knobs() {
-    static const Knobs k = [] {
-        Knobs x{4, 4, 4, 1, 3, 1, 3, 1};
-        auto cells = [](const char* name, int dflt) {
-            const char* e = getenv(name);
-            if (!e) e = getenv("DHTS_ARZ_C");
-            if (!e) return dflt;
-            const int c = atoi(e);
-            return (c == 1 || c == 2 || c == 4 || c == 8) ? c : dflt;
-        };
-        x.c_fwd = cells("DHTS_ARZ_C_FWD", 4); x.c_bwd = cells("DHTS_ARZ_C_BWD", 4);
-        if (const char* e = getenv("DHTS_ARZ_RING")) x.ring = atoi(e);      // 0 = register prefetch
-        if (const char* e = getenv("DHTS_ARZ_STAGE")) x.stage = atoi(e);    // 0 = per-thread stores
-        if (const char* e = getenv("DHTS_ARZ_XROW")) x.xrow = atoi(e);      // 0 = never store the interface outcomes
-        if (const char* e = getenv("DHTS_ARZ_UNI")) x.uni = atoi(e);         // 0: uniform-geometry calls run the per-lane-constant kernels
-        if (const char* e = getenv("DHTS_ARZ_MB_XFWD")) x.mb_xfwd = atoi(e); // forward kernel that also stores the interface outcomes
-        if (const char* e = getenv("DHTS_ARZ_MB_FWD")) x.mb_fwd = atoi(e);  // 3 (default) = 80-register forward kernel, 3 CTAs per SM: 384 vs 393 ms per pass (r2c A/B); 2 = 128 registers
-        return x;
-    }();
-    return k;
-}
-
-template <typename T> static int plan_reg(int B, int N, bool adj, RegPlan* p, bool xr = false) {
-    const int want = adj ? knobs().c_bwd : knobs().c_fwd;
+// Cells per thread and lanes per CTA, the same in both directions (the stored outcomes rely on it); no ring, no staging.
+template <typename T, typename Key> static int lane_shape(int B, int N, Plan<Key>* p) {
     int C = 1;
-    for (int c = 8; c > 1; c >>= 1)
-        if (want >= c && N % c == 0 && N / c >= 32) { C = c; break; }
+    for (int c = CELLS; c > 1; c >>= 1)
+        if (N % c == 0 && N / c >= 32) { C = c; break; }
     int tpl = N / C;
     while (tpl > 1024 / (C < 4 ? C : 4) && C < 8 && N % (2 * C) == 0) { C *= 2; tpl = N / C; }   // long lanes: wider chunks
     if (tpl > 1024 / (C < 4 ? C : 4)) return DHTS_ERR_UNSUPPORTED;
@@ -880,64 +875,137 @@ template <typename T> static int plan_reg(int B, int N, bool adj, RegPlan* p, bo
     int lpc = tpl >= target ? 1 : target / tpl;
     if (lpc > B) lpc = B;
     if (lpc < 1) lpc = 1;
-    p->C = C; p->lpc = lpc; p->threads = round32(lpc * tpl);
-    p->smem = shm_bytes<T>(lpc, p->threads / 32);
-    p->grid = (B + lpc - 1) / lpc;
-    // Adjoint with every state stored: shared-memory ring for the state rows (TMA bulk copies need 16-byte rows).
-    // Budget per CTA keeps two CTAs of the 128-register shape on an SM (227 KB usable, 1 KB reserved per CTA).
-    p->ring_ns = 0; p->mode = 1;
-    if (adj) {
-        const size_t stage = ((size_t)2 * lpc * N + (xr ? xrow_elems<T>(lpc, tpl, C) : 0)) * sizeof(T);
-        const size_t base = ring_offset<T>(lpc, p->threads / 32);
-        const size_t budget = (C > 1 ? 112 : 224) * (size_t)1024;
-        int ns = knobs().ring;
-        if (ns > 8) ns = 8;
-        while (ns >= 2 && base + ns * (stage + 8) > budget) ns--;
-        if (ns >= 2 && ((size_t)N * sizeof(T)) % 16 == 0 && (size_t)lpc * N * sizeof(T) < (1u << 19)) {
-            p->ring_ns = ns; p->mode = 0;
-            p->smem = base + ns * (stage + 8);
-        }
-    }
+    p->k.C = C; p->k.MB = C > 1 ? 2 : 1;
+    p->lpc = lpc; p->threads = round32(lpc * tpl); p->groups = (B + lpc - 1) / lpc;
+    p->ring_ns = 0; p->smem = shm_bytes<T>(lpc, p->threads / 32); p->rk = RollK();
     return DHTS_OK;
 }
 
-// MB is the register budget in units of "CTAs of 1024/min(C,4) threads per SM": 2 -> 128 registers (measured best
-// for every C > 1, profiles/r1e sweep), 1 -> 255.
-#define DHTS_C_DISPATCH(P, CALL)                                                                                   \
-    if ((P).C == 8) { CALL(8, 2) } else if ((P).C == 4) { CALL(4, 2) } else if ((P).C == 2) { CALL(2, 2) } else { CALL(1, 1) }
-#define CALL0(CC, MB) CALLM(CC, MB, 0)
-#define CALL1(CC, MB) CALLM(CC, MB, 1)
-#define CALL2(CC, MB) CALLM(CC, MB, 2)
-#define DHTS_CM_DISPATCH(P)                                                                                        \
-    if ((P).mode == 0) { DHTS_C_DISPATCH(P, CALL0) } else if ((P).mode == 1) { DHTS_C_DISPATCH(P, CALL1) } else { DHTS_C_DISPATCH(P, CALL2) }
-
-static int status_r() { return cudaGetLastError() == cudaSuccess ? DHTS_OK : DHTS_ERR_CUDA; }
-
-// Do the rollouts of this shape store the interface outcomes with the states (ckpt_mode 1)?  Yes when every state is stored
-// and the staged forward kernel and the ring adjoint both apply with the same thread -> cell mapping.  Callers ask
-// (dhts_arz_rollout_ckpt_elems_*), size `ckpt` accordingly and pass the mode to both calls.
-constexpr int NSF = 4;          // staging stages of the forward kernel
-template <typename T> static int ckpt_mode_plan(int B, int N, int K) {
-    if (!knobs().xrow || K != 1 || B <= 0 || N < 1) return 0;
-    RegPlan pf, pb;
-    // whole warps per lane (the outcomes are warp ballots, stored lane by lane)
-    if (plan_reg<T>(B, N, false, &pf) || pf.C <= 1 || ((size_t)N * sizeof(T)) % 16 != 0 || (N / pf.C) % 32 != 0) return 0;
-    const size_t stage = ((size_t)2 * pf.lpc * N + xrow_elems<T>(pf.lpc, N / pf.C, pf.C)) * sizeof(T);
-    if (ring_offset<T>(pf.lpc, pf.threads / 32, true) + NSF * stage > 112 * 1024) return 0;
-    if (plan_reg<T>(B, N, true, &pb, true) || pb.mode != 0 || pb.C != pf.C || pb.lpc != pf.lpc) return 0;
-    return 1;
+// Forward.  Every state stored (K == 1, no per-step ghosts) in 16-byte rows: the staging ring with TMA bulk stores, with the
+// interface outcomes behind the states when xmode == 1 (the outcomes are warp ballots, stored lane by lane: whole warps per
+// lane); the UNI instantiation for uniform geometry exists for the C = 4 kernel with outcomes, the bench's.  Otherwise
+// per-thread stores (TV: per-step ghosts).  K == 0: no checkpoints.
+template <typename T>
+static int fwd_plan(int B, int N, int K, int xmode, bool tv, bool uni, bool aligned, Plan<FwdKey>* p) {
+    const int rc = lane_shape<T>(B, N, p);
+    if (rc) return rc;
+    p->k.NS = 0; p->k.TV = tv; p->k.XR = p->k.UNI = false;
+    const int C = p->k.C, nwarp = p->threads / 32;
+    if (C > 1 && !aligned) return DHTS_ERR_UNSUPPORTED;          // callers step with the tiled kernels instead
+    if (K != 1 || tv || C == 1 || ((size_t)N * sizeof(T)) % 16 != 0) return DHTS_OK;
+    const bool xr = xmode == 1 && (N / C) % 32 == 0;
+    const size_t stage = ((size_t)2 * p->lpc * N + (xr ? xrow_elems<T>(p->lpc, N / C, C) : 0)) * sizeof(T);
+    const size_t smem = ring_offset<T>(p->lpc, nwarp, true) + NSF * stage;
+    if (smem > RING_BUDGET) return DHTS_OK;
+    p->k = FwdKey{C, C == 4 && smem <= MB3_BUDGET ? 3 : 2, NSF, false, xr, xr && uni && C == 4};
+    p->smem = smem;
+    p->rk = make_rollk<T>(B, N, C, p->lpc, nwarp, true, xr);
+    return DHTS_OK;
 }
+
+// Adjoint.  Every state stored (K == 1, no per-step ghosts or history) in 16-byte rows: MODE 0, the state ring filled by
+// TMA bulk loads, reading the stored outcomes when xmode == 1.  Otherwise MODE 1 (register prefetch; EXT: per-step ghosts /
+// history) or, with sparse checkpoints, MODE 2 (segment recompute).
+template <typename T>
+static int bwd_plan(int B, int N, int K, int xmode, bool ext, bool uni, bool aligned, Plan<BwdKey>* p) {
+    const int rc = lane_shape<T>(B, N, p);
+    if (rc) return rc;
+    p->k.MODE = K > 1 ? 2 : 1; p->k.EXT = ext; p->k.XR = p->k.UNI = false;
+    const int C = p->k.C, nwarp = p->threads / 32;
+    if (C > 1 && !aligned) return DHTS_ERR_UNSUPPORTED;
+    if (!ext) p->rk = make_rollk<T>(B, N, C, p->lpc, nwarp, false, false);
+    // a stage's two rows stay below the 2^20 bytes an mbarrier transaction count holds
+    if (K != 1 || ext || C == 1 || ((size_t)N * sizeof(T)) % 16 != 0 || (size_t)p->lpc * N * sizeof(T) >= (1u << 19))
+        return DHTS_OK;
+    const bool xr = xmode == 1;
+    const size_t stage = ((size_t)2 * p->lpc * N + (xr ? xrow_elems<T>(p->lpc, N / C, C) : 0)) * sizeof(T) + 8;  // + mbarrier
+    const size_t base = ring_offset<T>(p->lpc, nwarp);
+    int ns = RING_NS;
+    while (ns >= 2 && base + ns * stage > RING_BUDGET) ns--;
+    if (ns < 2) return DHTS_OK;
+    p->k = BwdKey{C, 2, 0, false, xr, xr && uni && C == 4};
+    p->ring_ns = ns; p->smem = base + ns * stage;
+    p->rk = make_rollk<T>(B, N, C, p->lpc, nwarp, false, xr);
+    return DHTS_OK;
+}
+
+// ckpt_mode 1: the rollouts of this shape store the interface outcomes with the states -- the forward plan is the staged
+// kernel with outcomes and the adjoint plan the ring with outcomes (same C and lpc: the rows written are the rows read).
+// Callers ask (dhts_arz_rollout_ckpt_elems_*), size `ckpt` accordingly and pass the mode to both calls.
+template <typename T> static bool outcomes_stored(int B, int N, int K, Plan<FwdKey>* f) {
+    Plan<BwdKey> b;
+    return B > 0 && N >= 1 && fwd_plan<T>(B, N, K, 1, false, false, true, f) == DHTS_OK && f->k.XR &&
+           bwd_plan<T>(B, N, K, 1, false, false, true, &b) == DHTS_OK && b.k.XR;
+}
+
+template <typename T> using FwdFn = decltype(&arz_rollout_fwd_reg_kernel<T, 1, 1, 0>);
+template <typename T> using BwdFn = decltype(&arz_rollout_bwd_reg_kernel<T, 1, 1, 1>);
+template <typename Key, typename Fn> struct Entry { Key k; Fn fn; };
+template <typename T, int C, int MB, int NS, bool TV = false, bool XR = false, bool UNI = false>
+static Entry<FwdKey, FwdFn<T>> fwd() { return {FwdKey{C, MB, NS, TV, XR, UNI}, arz_rollout_fwd_reg_kernel<T, C, MB, NS, TV, XR, UNI>}; }
+template <typename T, int C, int MB, int MODE, bool EXT = false, bool XR = false, bool UNI = false>
+static Entry<BwdKey, BwdFn<T>> bwd() { return {BwdKey{C, MB, MODE, EXT, XR, UNI}, arz_rollout_bwd_reg_kernel<T, C, MB, MODE, EXT, XR, UNI>}; }
+template <typename Key, typename Fn, size_t n> static Fn find(const Entry<Key, Fn> (&list)[n], const Key& k) {
+    for (const Entry<Key, Fn>& e : list)
+        if (e.k == k) return e.fn;
+    return nullptr;
+}
+
+template <typename T> static FwdFn<T> fwd_kernel(const FwdKey& k) {
+    static const Entry<FwdKey, FwdFn<T>> list[] = {
+        fwd<T, 1, 1, 0>(),                          // per-thread stores
+        fwd<T, 2, 2, 0>(),
+        fwd<T, 4, 2, 0>(),
+        fwd<T, 8, 2, 0>(),
+        fwd<T, 1, 1, 0, true>(),                    // per-step ghosts
+        fwd<T, 2, 2, 0, true>(),
+        fwd<T, 4, 2, 0, true>(),
+        fwd<T, 8, 2, 0, true>(),
+        fwd<T, 2, 2, NSF>(),                        // staged
+        fwd<T, 4, 3, NSF>(),
+        fwd<T, 8, 2, NSF>(),
+        fwd<T, 2, 2, NSF, false, true>(),           // staged with outcomes
+        fwd<T, 4, 3, NSF, false, true>(),
+        fwd<T, 8, 2, NSF, false, true>(),
+        fwd<T, 4, 3, NSF, false, true, true>(),     // staged with outcomes, uniform geometry
+    };
+    return find(list, k);
+}
+
+template <typename T> static BwdFn<T> bwd_kernel(const BwdKey& k) {
+    static const Entry<BwdKey, BwdFn<T>> list[] = {
+        bwd<T, 2, 2, 0>(),                          // ring
+        bwd<T, 4, 2, 0>(),
+        bwd<T, 8, 2, 0>(),
+        bwd<T, 2, 2, 0, false, true>(),             // ring with outcomes
+        bwd<T, 4, 2, 0, false, true>(),
+        bwd<T, 8, 2, 0, false, true>(),
+        bwd<T, 4, 2, 0, false, true, true>(),       // ring with outcomes, uniform geometry
+        bwd<T, 1, 1, 1>(),                          // register prefetch (C > 1 gets a ring, except fp32 C = 2 below)
+        bwd<T, 1, 1, 1, true>(),                    // per-step ghosts / history
+        bwd<T, 2, 2, 1, true>(),
+        bwd<T, 4, 2, 1, true>(),
+        bwd<T, 8, 2, 1, true>(),
+        bwd<T, 1, 1, 2>(),                          // segment recompute
+        bwd<T, 2, 2, 2>(),
+        bwd<T, 4, 2, 2>(),
+        bwd<T, 8, 2, 2>(),
+    };
+    if constexpr (std::is_same<T, float>::value) {  // fp32 C = 2 lanes with N % 4 == 2: rows that are not 16-byte sized
+        static const Entry<BwdKey, BwdFn<T>> fp32[] = {bwd<float, 2, 2, 1>()};
+        if (const BwdFn<T> fn = find(fp32, k)) return fn;
+    }
+    return find(list, k);
+}
+
 template <typename T> static long long ckpt_elems(int B, int N, int steps, int K, int* mode) {
     if (B < 0 || N < 1 || steps < 0 || K < 1) return -1;
-    const int m = ckpt_mode_plan<T>(B, N, K);
-    if (mode) *mode = m;
+    Plan<FwdKey> f;
+    const bool xr = outcomes_stored<T>(B, N, K, &f);
+    if (mode) *mode = xr;
     const long long S = (steps + K - 1) / K;
     long long n = S * 2 * (long long)B * N;
-    if (m) {
-        RegPlan pf;
-        plan_reg<T>(B, N, false, &pf);
-        n += ((long long)steps * B * (long long)xlane_bytes(N / pf.C, pf.C) + (long long)sizeof(T) - 1) / (long long)sizeof(T);
-    }
+    if (xr) n += ((long long)steps * B * (long long)xlane_bytes(N / f.k.C, f.k.C) + (long long)sizeof(T) - 1) / (long long)sizeof(T);
     return n;
 }
 
@@ -952,101 +1020,28 @@ static int rollout_fwd(const T* r0, const T* y0, const T* u0, const T* ghost, co
     const LaneK<T> kall = make_lanek<T>(uni ? umax_all : T(1), uni ? dx_all : T(1), dt);
     if (ckpt && K < 1) return DHTS_ERR_INVALID;
     if (xmode != 0 && xmode != 1) return DHTS_ERR_INVALID;
-    if (xmode == 1 && (!ckpt || ghost_t || ckpt_mode_plan<T>(B, N, K) != 1)) return DHTS_ERR_INVALID;
+    Plan<FwdKey> p;
+    if (xmode == 1 && (!ckpt || ghost_t || !outcomes_stored<T>(B, N, K, &p))) return DHTS_ERR_INVALID;
     if (B == 0) return DHTS_OK;
-    RegPlan p;
-    int rc = plan_reg<T>(B, N, false, &p);
+    const bool aligned = al16(r0) && al16(y0) && al16(u0) && al16(ckpt) && al16(rT) && al16(yT) && al16(uT);
+    int rc = fwd_plan<T>(B, N, ckpt ? K : 0, xmode, ghost_t != nullptr, uni, aligned, &p);
     if (rc) return rc;
-    if (p.C > 1 && !(al16(r0) && al16(y0) && al16(u0) && al16(ckpt) && al16(rT) && al16(yT) && al16(uT)))
-        return DHTS_ERR_UNSUPPORTED;          // callers step with the tiled kernels instead
-    if (K < 1) K = 1;
-    int grid = p.grid;
-    // every state stored: staging ring + TMA bulk stores when the rows are 16-byte sized and 4 stages fit
-    const size_t stage = (size_t)2 * p.lpc * N * sizeof(T);
-    const size_t base = ring_offset<T>(p.lpc, p.threads / 32, true);
-    bool staged = ckpt && K == 1 && p.C > 1 && ((size_t)N * sizeof(T)) % 16 == 0 && base + NSF * stage <= 112 * 1024;
-    if (knobs().stage == 0) staged = false;
-    if (xmode == 1) {   // staged, with the interface outcomes behind the states
-        if (!(al16(r0) && al16(y0) && al16(u0) && al16(ckpt))) return DHTS_ERR_UNSUPPORTED;
-        const size_t smem = base + NSF * (stage + xrow_elems<T>(p.lpc, N / p.C, p.C) * sizeof(T));
-#define CALL(CC, MB)                                                                                                   \
-    {                                                                                                                  \
-        cudaFuncSetAttribute(arz_rollout_fwd_reg_kernel<T, CC, MB, NSF, false, true>,                                  \
-                             cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);                                  \
-        arz_rollout_fwd_reg_kernel<T, CC, MB, NSF, false, true><<<grid, p.threads, smem, st>>>(                        \
-            r0, y0, u0, ghost, nullptr, dx, umax, kall, dt, B, N, steps, K, p.lpc, make_rollk<T>(B, N, CC, p.lpc, p.threads / 32, true, true), ckpt, rT, yT, uT, flags); \
-    }
-        // 80 registers, three CTAs per SM by default (391 vs 405 ms per pass, r2u A/B); DHTS_ARZ_MB_XFWD=2: 128 registers
-#define CALLU(CC, MB)                                                                                                  \
-    {                                                                                                                  \
-        cudaFuncSetAttribute(arz_rollout_fwd_reg_kernel<T, CC, MB, NSF, false, true, true>,                            \
-                             cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);                                  \
-        arz_rollout_fwd_reg_kernel<T, CC, MB, NSF, false, true, true><<<grid, p.threads, smem, st>>>(                  \
-            r0, y0, u0, ghost, nullptr, dx, umax, kall, dt, B, N, steps, K, p.lpc, make_rollk<T>(B, N, CC, p.lpc, p.threads / 32, true, true), ckpt, rT, yT, uT, flags); \
-    }
-        const bool mb3 = knobs().mb_xfwd == 3 && smem <= 74 * 1024;
-        if (p.C == 8) { CALL(8, 2) }
-        else if (p.C == 4) { if (uni && knobs().uni) { if (mb3) { CALLU(4, 3) } else { CALLU(4, 2) } } else if (mb3) { CALL(4, 3) } else { CALL(4, 2) } }
-        else { CALL(2, 2) }
-#undef CALL
-#undef CALLU
-        return status_r();
-    }
-    if (ghost_t) {      // per-step ghosts: the variant with per-thread checkpoint stores
-#define CALL(CC, MB) arz_rollout_fwd_reg_kernel<T, CC, MB, 0, true><<<grid, p.threads, p.smem, st>>>(r0, y0, u0, nullptr, ghost_t, dx, umax, kall, dt, B, N, steps, K, p.lpc, RollK(), ckpt, rT, yT, uT, flags);
-        DHTS_C_DISPATCH(p, CALL)
-#undef CALL
-    } else if (staged) {
-        const size_t smem = base + NSF * stage;
-#define CALL(CC, MB)                                                                                                   \
-    {                                                                                                                  \
-        if (smem > 48 * 1024)                                                                                          \
-            cudaFuncSetAttribute(arz_rollout_fwd_reg_kernel<T, CC, MB, NSF>,                                           \
-                                 cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);                              \
-        arz_rollout_fwd_reg_kernel<T, CC, MB, NSF><<<grid, p.threads, smem, st>>>(                                     \
-            r0, y0, u0, ghost, nullptr, dx, umax, kall, dt, B, N, steps, K, p.lpc, make_rollk<T>(B, N, CC, p.lpc, p.threads / 32, true, false), ckpt, rT, yT, uT, flags); \
-    }
-        if (p.C == 4 && knobs().mb_fwd == 3 && base + NSF * stage <= 74 * 1024) { CALL(4, 3) } else { DHTS_C_DISPATCH(p, CALL) }
-#undef CALL
-    } else {
-#define CALL(CC, MB) arz_rollout_fwd_reg_kernel<T, CC, MB, 0><<<grid, p.threads, p.smem, st>>>(r0, y0, u0, ghost, nullptr, dx, umax, kall, dt, B, N, steps, K, p.lpc, RollK(), ckpt, rT, yT, uT, flags);
-        DHTS_C_DISPATCH(p, CALL)
-#undef CALL
-    }
-    return status_r();
-}
-
-// adjoint mode (see the kernel): recompute when K > 1, else the ring when it was planned and applies
-template <typename T> static void set_mode(RegPlan* p, int K, bool ring_ok) {
-    if (K == 1 && ring_ok && p->ring_ns > 0 && p->C > 1) { p->mode = 0; return; }
-    p->ring_ns = 0; p->mode = K > 1 ? 2 : 1;
-    p->smem = shm_bytes<T>(p->lpc, p->threads / 32);
-}
-
-template <typename T> static int bwd_grid_r(const RegPlan& p) {
-    int occ = 0;
-#define CALLM(CC, MB, MD)                                                                                              \
-    {                                                                                                                  \
-        if (p.smem > 48 * 1024)                                                                                        \
-            cudaFuncSetAttribute(arz_rollout_bwd_reg_kernel<T, CC, MB, MD>,                                            \
-                                 cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem);                            \
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, arz_rollout_bwd_reg_kernel<T, CC, MB, MD>, p.threads,      \
-                                                      p.smem);                                                         \
-    }
-    DHTS_CM_DISPATCH(p)
-#undef CALLM
-    if (occ < 1) occ = 1;
-    long long g = (long long)sm_count_r() * occ;
-    return (int)(g < p.grid ? g : p.grid);
+    const FwdFn<T> kernel = fwd_kernel<T>(p.k);
+    if (!kernel) return DHTS_ERR_CUDA;            // a plan without an instantiation: nothing to launch
+    if ((rc = set_smem(kernel, p.smem))) return rc;
+    kernel<<<p.groups, p.threads, p.smem, st>>>(r0, y0, u0, ghost_t ? nullptr : ghost, ghost_t, dx, umax, kall, dt, B, N, steps,
+                                               K < 1 ? 1 : K, p.lpc, p.rk, ckpt, rT, yT, uT, flags);
+    return launch_status();
 }
 
 template <typename T> static long long rollout_scratch_elems(int B, int N, int K) {
-    RegPlan p;
+    Plan<BwdKey> p;
     if (B <= 0) return 0;
-    if (K < 1 || plan_reg<T>(B, N, true, &p)) return -1;
+    if (K < 1 || bwd_plan<T>(B, N, K, 0, false, false, true, &p)) return -1;
     if (K == 1) return 0;                      // every state comes from the forward pass: nothing to stash
-    set_mode<T>(&p, K, false);
-    return (long long)bwd_grid_r<T>(p) * K * 2 * p.lpc * N;
+    int grid = 1;
+    if (persistent_grid(bwd_kernel<T>(p.k), p.threads, p.smem, p.groups, &grid)) return -1;
+    return (long long)grid * K * 2 * p.lpc * N;
 }
 
 template <typename T>
@@ -1065,71 +1060,22 @@ static int rollout_bwd(const T* ckpt, const T* u0, const T* ghost, const T* ghos
     if (g_uT && (!rT || !yT)) return DHTS_ERR_INVALID;
     if (xmode != 0 && xmode != 1) return DHTS_ERR_INVALID;
     if (B == 0) return DHTS_OK;
-    if (xmode == 1) {   // the interface outcomes were stored with the states: ring adjoint without the case tree
-        if (ext || ckpt_mode_plan<T>(B, N, K) != 1) return DHTS_ERR_INVALID;
-        RegPlan p;
-        int rc = plan_reg<T>(B, N, true, &p, true);
-        if (rc) return rc;
-        if (!(al16(ckpt) && al16(u0) && al16(g_r0) && al16(g_y0))) return DHTS_ERR_UNSUPPORTED;
-        int occ = 0, grid = 1;
-#define CALL(CC, MB)                                                                                                   \
-    {                                                                                                                  \
-        cudaFuncSetAttribute(arz_rollout_bwd_reg_kernel<T, CC, MB, 0, false, true>,                                       \
-                             cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem);                                \
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, arz_rollout_bwd_reg_kernel<T, CC, MB, 0, false, true>,        \
-                                                      p.threads, p.smem);                                              \
-        const long long g = (long long)sm_count_r() * (occ < 1 ? 1 : occ);                                             \
-        grid = (int)(g < p.grid ? g : p.grid);                                                                         \
-        arz_rollout_bwd_reg_kernel<T, CC, MB, 0, false, true><<<grid, p.threads, p.smem, st>>>(                           \
-            ckpt, u0, ghost, nullptr, nullptr, nullptr, dx, umax, kall, dt, B, N, steps, K, p.lpc, rT, yT, g_rT, g_yT, g_uT, \
-            scratch, g_r0, g_y0, g_ghost, flags, p.ring_ns, make_rollk<T>(B, N, CC, p.lpc, p.threads / 32, false, true)); \
-    }
-#define CALLU(CC, MB)                                                                                                  \
-    {                                                                                                                  \
-        cudaFuncSetAttribute(arz_rollout_bwd_reg_kernel<T, CC, MB, 0, false, true, true>,                              \
-                             cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem);                                \
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, arz_rollout_bwd_reg_kernel<T, CC, MB, 0, false, true, true>, \
-                                                      p.threads, p.smem);                                              \
-        const long long g = (long long)sm_count_r() * (occ < 1 ? 1 : occ);                                             \
-        grid = (int)(g < p.grid ? g : p.grid);                                                                         \
-        arz_rollout_bwd_reg_kernel<T, CC, MB, 0, false, true, true><<<grid, p.threads, p.smem, st>>>(                  \
-            ckpt, u0, ghost, nullptr, nullptr, nullptr, dx, umax, kall, dt, B, N, steps, K, p.lpc, rT, yT, g_rT, g_yT, g_uT, \
-            scratch, g_r0, g_y0, g_ghost, flags, p.ring_ns, make_rollk<T>(B, N, CC, p.lpc, p.threads / 32, false, true)); \
-    }
-        if (p.C == 8) { CALL(8, 2) } else if (p.C == 4) { if (uni && knobs().uni) { CALLU(4, 2) } else { CALL(4, 2) } } else { CALL(2, 2) }
-#undef CALL
-#undef CALLU
-        return status_r();
-    }
-    RegPlan p;
-    int rc = plan_reg<T>(B, N, true, &p);
+    Plan<FwdKey> f;
+    if (xmode == 1 && (ext || !outcomes_stored<T>(B, N, K, &f))) return DHTS_ERR_INVALID;
+    // the ring with outcomes uses no scratch
+    const bool aligned = al16(ckpt) && al16(u0) && al16(g_r0) && al16(g_y0) && (xmode == 1 || (al16(scratch) && al16(g_hist)));
+    Plan<BwdKey> p;
+    int rc = bwd_plan<T>(B, N, K, xmode, ext, uni, aligned, &p);
     if (rc) return rc;
-    if (p.C > 1 && !(al16(ckpt) && al16(u0) && al16(scratch) && al16(g_r0) && al16(g_y0))) return DHTS_ERR_UNSUPPORTED;
-    set_mode<T>(&p, K, al16(ckpt) && !ext);
-    if (ext && p.C > 1 && !al16(g_hist)) return DHTS_ERR_UNSUPPORTED;
-    int grid = bwd_grid_r<T>(p);
+    const BwdFn<T> kernel = bwd_kernel<T>(p.k);
+    if (!kernel) return DHTS_ERR_CUDA;            // a plan without an instantiation: nothing to launch
+    int grid = 1;
+    if ((rc = persistent_grid(kernel, p.threads, p.smem, p.groups, &grid))) return rc;
     if (K > 1 && (long long)grid * K * 2 * p.lpc * N > scratch_elems) return DHTS_ERR_INVALID;
-    if (ext) {
-#define CALL(CC, MB)                                                                                                   \
-    arz_rollout_bwd_reg_kernel<T, CC, MB, 1, true><<<grid, p.threads, p.smem, st>>>(                                   \
-        ckpt, u0, ghost_t ? nullptr : ghost, ghost_t, g_hist, g_ghost_t, dx, umax, kall, dt, B, N, steps, K, p.lpc, rT, yT,  \
-        g_rT, g_yT, g_uT, scratch, g_r0, g_y0, g_ghost, flags, 0, RollK());
-        DHTS_C_DISPATCH(p, CALL)
-#undef CALL
-        return status_r();
-    }
-#define CALLM(CC, MB, MD)                                                                                              \
-    {                                                                                                                  \
-        if (p.smem > 48 * 1024)                                                                                        \
-            cudaFuncSetAttribute(arz_rollout_bwd_reg_kernel<T, CC, MB, MD>,                                            \
-                                 cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem);                            \
-        arz_rollout_bwd_reg_kernel<T, CC, MB, MD><<<grid, p.threads, p.smem, st>>>(                                    \
-            ckpt, u0, ghost, nullptr, nullptr, nullptr, dx, umax, kall, dt, B, N, steps, K, p.lpc, rT, yT, g_rT, g_yT, g_uT, \
-            scratch, g_r0, g_y0, g_ghost, flags, p.ring_ns, make_rollk<T>(B, N, CC, p.lpc, p.threads / 32, false, false)); \
-    }
-    DHTS_CM_DISPATCH(p)
-#undef CALLM
-    return status_r();
+    kernel<<<grid, p.threads, p.smem, st>>>(ckpt, u0, ghost_t ? nullptr : ghost, ghost_t, g_hist, ext ? g_ghost_t : nullptr, dx,
+                                           umax, kall, dt, B, N, steps, K, p.lpc, rT, yT, g_rT, g_yT, g_uT, scratch, g_r0, g_y0,
+                                           g_ghost, flags, p.ring_ns, p.rk);
+    return launch_status();
 }
 
 }  // namespace dhts

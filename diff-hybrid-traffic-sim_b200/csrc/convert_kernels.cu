@@ -136,8 +136,6 @@ __global__ void c2m_bwd_kernel(const T* __restrict__ p_head, const T* __restrict
     g_p[j] = gp; g_v[j] = gv; g_a[j] = ga;
 }
 
-static int cv_status() { return cudaGetLastError() == cudaSuccess ? DHTS_OK : DHTS_ERR_CUDA; }
-
 }  // namespace dhts
 
 #define DHTS_CV_API(SUF, T)                                                                                            \
@@ -150,7 +148,7 @@ static int cv_status() { return cudaGetLastError() == cudaSuccess ? DHTS_OK : DH
         dhts::m2c_fwd_kernel<T><<<(J + dhts::CV_BLOCK - 1) / dhts::CV_BLOCK, dhts::CV_BLOCK, 0,                        \
                                   (cudaStream_t)stream>>>(cap, r_last, u_last, free_space, veh_len, dt, J, cap_out,    \
                                                           spawn, v_new, a_new);                                        \
-        return dhts::cv_status();                                                                                      \
+        return dhts::launch_status();                                                                                  \
     }                                                                                                                  \
     DHTS_EXPORT int dhts_m2c_bwd_##SUF(const T* r_last, const T* u_last, const int* spawn, T dt, int J,                \
                                        const T* g_cap_out, const T* g_v_new, const T* g_a_new, T* g_cap,               \
@@ -162,7 +160,7 @@ static int cv_status() { return cudaGetLastError() == cudaSuccess ? DHTS_OK : DH
         dhts::m2c_bwd_kernel<T><<<(J + dhts::CV_BLOCK - 1) / dhts::CV_BLOCK, dhts::CV_BLOCK, 0,                        \
                                   (cudaStream_t)stream>>>(r_last, u_last, spawn, dt, J, g_cap_out, g_v_new, g_a_new,   \
                                                           g_cap, g_r_last, g_u_last);                                  \
-        return dhts::cv_status();                                                                                      \
+        return dhts::launch_status();                                                                                  \
     }                                                                                                                  \
     DHTS_EXPORT int dhts_c2m_fwd_##SUF(const T* p_head, const T* v_head, const T* a_head, const T* len_head,           \
                                        const T* lane_len, const T* r, const T* y, const T* u, const T* dx,             \
@@ -175,7 +173,7 @@ static int cv_status() { return cudaGetLastError() == cudaSuccess ? DHTS_OK : DH
         dhts::c2m_fwd_kernel<T><<<(J + dhts::CV_BLOCK - 1) / dhts::CV_BLOCK, dhts::CV_BLOCK, 0,                        \
                                   (cudaStream_t)stream>>>(p_head, v_head, a_head, len_head, lane_len, r, y, u, dx,     \
                                                           umax, J, N, r_out, y_out, u_out, absorbed, ntouched);        \
-        return dhts::cv_status();                                                                                      \
+        return dhts::launch_status();                                                                                  \
     }                                                                                                                  \
     DHTS_EXPORT int dhts_c2m_bwd_##SUF(const T* p_head, const T* v_head, const T* a_head, const T* len_head,           \
                                        const T* lane_len, const T* r_out, const T* dx, const T* umax,                  \
@@ -190,7 +188,7 @@ static int cv_status() { return cudaGetLastError() == cudaSuccess ? DHTS_OK : DH
                                   (cudaStream_t)stream>>>(p_head, v_head, a_head, len_head, lane_len, r_out, dx, umax, \
                                                           ntouched, J, N, g_r_out, g_y_out, g_u_out, g_p, g_v, g_a,    \
                                                           g_r, g_y, g_u);                                              \
-        return dhts::cv_status();                                                                                      \
+        return dhts::launch_status();                                                                                  \
     }
 
 DHTS_CV_API(f64, double)

@@ -365,16 +365,10 @@ idm_rollout_bwd_kernel(const T* __restrict__ ckpt, const T* __restrict__ params,
 
 // ------------------------------------------------------------------ host side
 
-static int last_status_idm() { return cudaGetLastError() == cudaSuccess ? DHTS_OK : DHTS_ERR_CUDA; }
-
 static int idm_grid(int L) {
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    if (sms <= 0) sms = 148;
     int warps_per_block = IDM_ROLL_BLOCK / 32;
     long long want = ((long long)L + warps_per_block - 1) / warps_per_block;
-    long long cap = (long long)sms * 16;
+    long long cap = (long long)sm_count() * 16;
     return (int)(want < cap ? (want < 1 ? 1 : want) : cap);
 }
 
@@ -386,7 +380,7 @@ static int idm_step_fwd(const T* p, const T* v, const T* params, const int* lane
     if (V == 0) return DHTS_OK;
     idm_step_fwd_kernel<T><<<(V + IDM_BLOCK - 1) / IDM_BLOCK, IDM_BLOCK, 0, st>>>(p, v, params, lane_off, veh_lane, head,
                                                                                   dt, V, np_, nv_, vflags, flags);
-    return last_status_idm();
+    return launch_status();
 }
 
 // g_params NULL: the state adjoint only (dhts_idm_step_bwd_*)
@@ -398,7 +392,7 @@ static int idm_step_bwd(const T* p, const T* v, const T* params, const int* lane
         L < 0)
         return DHTS_ERR_INVALID;
     if (g_head && L > 0) idm_zero_empty_head_kernel<T><<<(L + 255) / 256, 256, 0, st>>>(lane_off, L, g_head);
-    if (V == 0) return last_status_idm();
+    if (V == 0) return launch_status();
     const int grid = (V + IDM_BLOCK - 1) / IDM_BLOCK;
     if (g_params)
         idm_step_bwd_kernel<T, true><<<grid, IDM_BLOCK, 0, st>>>(p, v, params, lane_off, veh_lane, head, dt, V, g_np, g_nv,
@@ -406,7 +400,7 @@ static int idm_step_bwd(const T* p, const T* v, const T* params, const int* lane
     else
         idm_step_bwd_kernel<T, false><<<grid, IDM_BLOCK, 0, st>>>(p, v, params, lane_off, veh_lane, head, dt, V, g_np, g_nv,
                                                                   g_p, g_v, g_head, flags, nullptr);
-    return last_status_idm();
+    return launch_status();
 }
 
 #define DHTS_VPT_DISPATCH(max_lane, CALL)        \
@@ -430,7 +424,7 @@ static int idm_rollout_fwd(const T* p0, const T* v0, const T* params, const int*
                     else idm_rollout_fwd_kernel<T, VPT, false><<<grid, IDM_ROLL_BLOCK, 0, st>>>(p0, v0, params, lane_off, head, nullptr, dt, V, L, steps, K, ckpt, pT, vT, flags); }
     DHTS_VPT_DISPATCH(max_lane, CALL)
 #undef CALL
-    return last_status_idm();
+    return launch_status();
 }
 
 // g_params NULL: the state adjoint only (dhts_idm_rollout_bwd_*)
@@ -452,7 +446,7 @@ static int idm_rollout_bwd(const T* ckpt, const T* params, const int* lane_off, 
     DHTS_VPT_DISPATCH(max_lane, CALL)
 #undef CALL
 #undef LAUNCH
-    return last_status_idm();
+    return launch_status();
 }
 
 }  // namespace dhts
@@ -514,7 +508,7 @@ DHTS_EXPORT int dhts_csr_expand(const int* lane_off, int L, int* veh_lane, void*
     int blocks = (L + 7) / 8;
     if (blocks > 148 * 8) blocks = 148 * 8;
     dhts::csr_expand_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(lane_off, L, veh_lane);
-    return cudaGetLastError() == cudaSuccess ? DHTS_OK : DHTS_ERR_CUDA;
+    return dhts::launch_status();
 }
 
 DHTS_EXPORT int dhts_idm_rollout_max_ckpt_every(void) { return dhts::IDM_KMAX; }

@@ -984,21 +984,12 @@ __global__ void __launch_bounds__(TMAX, TMAX <= 192 ? 2 : 1) hyb_rollout_bwd_ker
 }
 
 // ------------------------------------------------------------------------------------------------ host side
-static int hyb_sm_count() {
-    static int nsm = 0;
-    if (!nsm) {
-        int dev = 0; cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev);
-        if (nsm <= 0) nsm = 148;
-    }
-    return nsm;
-}
 // Few replicas (a CTA's step time is what counts): one thread per interface of the macro lanes, and at least one per (side,
 // lane) plus one per micro lane.  Many replicas (several CTAs per SM hide each other's barriers): half as many, looping.
 template <typename T> static int hyb_threads(const HybArgs<T>& a) {
     const int NI = a.n.NC + (a.n.L - a.ML), sides = 2 * a.n.L + a.ML;
     int w = NI > sides ? NI : sides;
-    if (a.n.R > hyb_sm_count()) w = (w + 1) / 2;
+    if (a.n.R > sm_count()) w = (w + 1) / 2;
     int t = (w + 31) / 32 * 32;
     return t > HYB_THREADS_MAX ? HYB_THREADS_MAX : (t < 32 ? 32 : t);
 }
@@ -1038,20 +1029,6 @@ template <typename T> static int hyb_check(const HybArgs<T>& a) {
     if (n.mode != 0 && n.mode != 1) return DHTS_ERR_INVALID;
     if (a.NP < 1 || !a.par_tab || !(a.vlen > T(0))) return DHTS_ERR_INVALID;
     if (a.src && (n.mode != 1 || !a.rnd || a.NRAND < 0 || (a.KS > 0 && !a.spawn_route))) return DHTS_ERR_INVALID;
-    return DHTS_OK;
-}
-
-template <typename K> static int hyb_launch_cfg(K kernel, size_t smem, int threads, int R, int* grid) {
-    if (smem > 227 * 1024) return DHTS_ERR_UNSUPPORTED;
-    if (smem > 48 * 1024 && cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
-        cudaGetLastError();
-        return DHTS_ERR_CUDA;
-    }
-    int occ = 0;
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, threads, smem);
-    if (occ < 1) occ = 1;
-    const long long g = (long long)hyb_sm_count() * occ;
-    *grid = (int)(g < R ? g : R);
     return DHTS_OK;
 }
 
@@ -1104,12 +1081,12 @@ static HybArgs<T> hyb_args(const dhts_hyb_topology* tp, const T* dx, const T* la
         const int threads = dhts::hyb_threads(a);                                                                  \
         const size_t smem = dhts::hyb_smem<T>(a, false);                                                               \
         int grid = 1;                                                                                                  \
-        rc = dhts::hyb_launch_cfg(dhts::hyb_rollout_fwd_kernel<T>, smem, threads, R, &grid);                           \
+        rc = dhts::persistent_grid(dhts::hyb_rollout_fwd_kernel<T>, threads, smem, R, &grid);                          \
         if (rc) return rc;                                                                                             \
         dhts::hyb_rollout_fwd_kernel<T><<<grid, threads, smem, (cudaStream_t)stream>>>(a, r0, y0, u0, ueq0, own0,      \
                                                                                          aux0, hist, own_hist,        \
                                                                                          aux_hist, head_hist, flags);  \
-        return cudaGetLastError() == cudaSuccess ? DHTS_OK : DHTS_ERR_CUDA;                                            \
+        return dhts::launch_status();                                                                                  \
     }                                                                                                                  \
     DHTS_EXPORT int dhts_hyb_rollout_bwd_##SUF(const dhts_hyb_topology* topo, const T* dx, const T* lane_len,          \
                                                const int* route, int route_per_replica, const int* spawn_route,        \
@@ -1135,19 +1112,19 @@ static HybArgs<T> hyb_args(const dhts_hyb_topology* tp, const T* dx, const T* la
         if (smem > 227 * 1024) { a.prefetch = 0; smem = dhts::hyb_smem<T>(a, true); }                                  \
         int grid = 1;                                                                                                  \
         if (threads <= 192) {                                                                                          \
-            rc = dhts::hyb_launch_cfg(dhts::hyb_rollout_bwd_kernel<T, 192>, smem, threads, R, &grid);                  \
+            rc = dhts::persistent_grid(dhts::hyb_rollout_bwd_kernel<T, 192>, threads, smem, R, &grid);                 \
             if (rc) return rc;                                                                                         \
             dhts::hyb_rollout_bwd_kernel<T, 192><<<grid, threads, smem, (cudaStream_t)stream>>>(                       \
                 a, hist, own_hist, aux_hist, g_states, g_aux, g_r0, g_y0, g_u0, g_own0, g_sig, g_incoming, g_aux0,     \
                 flags);                                                                                                \
         } else {                                                                                                       \
-            rc = dhts::hyb_launch_cfg(dhts::hyb_rollout_bwd_kernel<T, dhts::HYB_THREADS_MAX>, smem, threads, R, &grid); \
+            rc = dhts::persistent_grid(dhts::hyb_rollout_bwd_kernel<T, dhts::HYB_THREADS_MAX>, threads, smem, R, &grid); \
             if (rc) return rc;                                                                                         \
             dhts::hyb_rollout_bwd_kernel<T, dhts::HYB_THREADS_MAX><<<grid, threads, smem, (cudaStream_t)stream>>>(     \
                 a, hist, own_hist, aux_hist, g_states, g_aux, g_r0, g_y0, g_u0, g_own0, g_sig, g_incoming, g_aux0,     \
                 flags);                                                                                                \
         }                                                                                                              \
-        return cudaGetLastError() == cudaSuccess ? DHTS_OK : DHTS_ERR_CUDA;                                            \
+        return dhts::launch_status();                                                                                  \
     }
 
 DHTS_HYB_API(f64, double)

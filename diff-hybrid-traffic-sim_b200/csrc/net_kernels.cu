@@ -30,7 +30,6 @@
 // ghosts, runs the flux-difference adjoint over its cells, pulls the ghost adjoint back through from_r_u and the
 // blend, and publishes (d green, d signal) per side in shared memory; after one barrier each lane GATHERS what its
 // neighbours published for its edge cells and for its signal (fixed order: deterministic, no atomics).
-#include <cstdlib>
 #include <cuda_pipeline.h>
 #include "dhts_net_if.cuh"
 
@@ -319,26 +318,16 @@ __global__ void __launch_bounds__(MAXTH, MINB) net_rollout_bwd_kernel(NetArgs<T>
 }
 
 // ------------------------------------------------------------------------------------------------ host side
-static int net_sm_count() {
-    static int n = 0;
-    if (!n) {
-        int dev = 0; cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
-        if (n <= 0) n = 148;
-    }
-    return n;
-}
 // Few replicas (latency-bound: a CTA's step time is what counts): one thread per interface, NC + L of them, up to 512.
 // Many replicas (throughput-bound: several CTAs per SM hide each other's barriers): a fraction of that, each thread looping --
 // a third for the forward kernel (on the ITSCP grid 2 L = NC = 288 and NI = 432 are then 2, 2 and 3 nearly full iterations of
 // 160 threads: 16.1 instead of 17.9 ms at 2048 replicas, r3w), half for the adjoint (three 80-register CTAs per SM; a third
 // measured 43.2 instead of 41.5 ms).
+constexpr int NET_DIV_FWD = 3, NET_DIV_BWD = 2;
 static int net_threads(int L, int NC, int R, bool adj) {
     int ni = NC + L;
-    static const int divf = [] { const char* e = getenv("DHTS_NET_DIV_FWD"); const int d = e ? atoi(e) : 3; return d >= 1 && d <= 8 ? d : 3; }();
-    static const int divb = [] { const char* e = getenv("DHTS_NET_DIV_BWD"); const int d = e ? atoi(e) : 2; return d >= 1 && d <= 8 ? d : 2; }();
-    const int div = adj ? divb : divf;
-    if (R > net_sm_count()) ni = (ni + div - 1) / div;
+    const int div = adj ? NET_DIV_BWD : NET_DIV_FWD;
+    if (R > sm_count()) ni = (ni + div - 1) / div;
     int t = (ni + 31) / 32 * 32;
     return t > 512 ? 512 : (t < 32 ? 32 : t);
 }
@@ -354,20 +343,6 @@ static int net_check(const NetArgs<T>& a) {
     return DHTS_OK;
 }
 
-template <typename T, typename K> static int net_launch_cfg(K kernel, size_t smem, int threads, int R, int* grid) {
-    if (smem > 227 * 1024) return DHTS_ERR_UNSUPPORTED;
-    if (smem > 48 * 1024 && cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
-        cudaGetLastError();
-        return DHTS_ERR_CUDA;
-    }
-    int occ = 0;
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, threads, smem);
-    if (occ < 1) occ = 1;
-    long long g = (long long)net_sm_count() * occ;
-    *grid = (int)(g < R ? g : R);
-    return DHTS_OK;
-}
-
 template <typename T>
 static int net_fwd(const NetArgs<T>& a, const T* r0, const T* y0, const T* u0, const T* own0, T* hist, T* ownh, T* reward,
                    int* flags, cudaStream_t st) {
@@ -378,10 +353,10 @@ static int net_fwd(const NetArgs<T>& a, const T* r0, const T* y0, const T* u0, c
     const int threads = net_threads(a.L, a.NC, a.R, false);
     const size_t smem = net_smem<T>(a.L, a.NC, a.n_own, false, threads);
     int grid = 1;
-    rc = net_launch_cfg<T>(net_rollout_fwd_kernel<T>, smem, threads, a.R, &grid);
+    rc = persistent_grid(net_rollout_fwd_kernel<T>, threads, smem, a.R, &grid);
     if (rc) return rc;
     net_rollout_fwd_kernel<T><<<grid, threads, smem, st>>>(a, r0, y0, u0, own0, hist, ownh, reward, flags);
-    return cudaGetLastError() == cudaSuccess ? DHTS_OK : DHTS_ERR_CUDA;
+    return launch_status();
 }
 
 template <typename T>
@@ -394,19 +369,18 @@ static int net_bwd(const NetArgs<T>& a, const T* hist, const T* ownh, const T* g
     const int threads = net_threads(a.L, a.NC, a.R, true);
     const size_t smem = net_smem<T>(a.L, a.NC, a.n_own, true, threads);
     int grid = 1;
-    static const bool occ3 = [] { const char* e = getenv("DHTS_NET_BWD_MINB"); return !e || atoi(e) != 1; }();
-    if (threads <= 256 && a.R > net_sm_count() && occ3) {
-        rc = net_launch_cfg<T>(net_rollout_bwd_kernel<T, 256, 3>, smem, threads, a.R, &grid);
+    if (threads <= 256 && a.R > sm_count()) {       // many replicas: 80 registers, three CTAs per SM (44.8 -> 41.2 ms)
+        rc = persistent_grid(net_rollout_bwd_kernel<T, 256, 3>, threads, smem, a.R, &grid);
         if (rc) return rc;
         net_rollout_bwd_kernel<T, 256, 3><<<grid, threads, smem, st>>>(a, hist, ownh, g_states, g_reward, g_r0, g_y0, g_u0, g_own0,
                                                                        g_sig, g_inc, flags);
     } else {
-        rc = net_launch_cfg<T>(net_rollout_bwd_kernel<T, 512, 1>, smem, threads, a.R, &grid);
+        rc = persistent_grid(net_rollout_bwd_kernel<T, 512, 1>, threads, smem, a.R, &grid);
         if (rc) return rc;
         net_rollout_bwd_kernel<T, 512, 1><<<grid, threads, smem, st>>>(a, hist, ownh, g_states, g_reward, g_r0, g_y0, g_u0, g_own0,
                                                                        g_sig, g_inc, flags);
     }
-    return cudaGetLastError() == cudaSuccess ? DHTS_OK : DHTS_ERR_CUDA;
+    return launch_status();
 }
 
 template <typename T> static NetArgs<T> net_args(const dhts_net_topology* tp, const int* route, int route_per_replica, T umax, T dt,

@@ -114,7 +114,7 @@ int dhts_arz_step_bwd_f32(const float* r_pad, const float* y_pad, const float* u
  *                          kernels apply); callers pass that mode to both calls (0 is always accepted)
  *   rT, yT, uT [B][N]      final state, uT = compute_u(rT, yT)
  * Limits of the fused kernels: a lane must fit one CTA -- N <= 1024 cells in general (one or two cells per thread),
- * N <= 2048 when N is a multiple of 8 (256 threads x 8 cells; plan_reg in csrc/arz_rollout.cu) -- and with more than
+ * N <= 2048 when N is a multiple of 8 (256 threads x 8 cells; lane_shape in csrc/arz_rollout.cu) -- and with more than
  * one cell per thread every array must be 16-byte aligned.  Otherwise the call returns DHTS_ERR_UNSUPPORTED and enqueues nothing; the host then chains
  * `steps` launches of the one-step entry points (dhts_b200.functional.arz_rollout does).  The IDM rollouts take lanes
  * of at most dhts_idm_rollout_max_lane() = 256 vehicles and checkpoint intervals up to

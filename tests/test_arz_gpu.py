@@ -233,41 +233,100 @@ def test_rollout_uniform_geometry_equals_per_lane_arrays(dev, dtype, B, N, T, K)
         assert torch.equal(x, y)
 
 
+# Launch routes of the fused rollout, reached through the inputs alone: (K, uniform geometry, state history) -> the template
+# arguments of the forward kernel (C, MB, NS, TV, XR, UNI) and of the adjoint kernel (C, MB, MODE, EXT, XR, UNI) that must run.
+# Per dtype where the two differ (fp64 rows of 2048 cells do not fit the staging ring; fp32 rows of 98 cells are not
+# 16-byte sized).
+_F, _T = False, True
+_ROUTES = {
+    # 1024 cells, 701 lanes: more lane groups than adjoint CTAs; stored outcomes (with and without per-lane geometry), the
+    # state history (staged forward, EXT adjoint) and sparse checkpoints (per-thread stores, recompute)
+    (701, 1024, 7): [
+        ((1, True, False), {"*": ((4, 3, 4, _F, _T, _T), (4, 2, 0, _F, _T, _T))}),
+        ((1, False, False), {"*": ((4, 3, 4, _F, _T, _F), (4, 2, 0, _F, _T, _F))}),
+        ((1, True, True), {"*": ((4, 3, 4, _F, _F, _F), (4, 2, 1, _T, _F, _F))}),
+        ((8, True, False), {"*": ((4, 2, 0, _F, _F, _F), (4, 2, 2, _F, _F, _F))}),
+    ],
+    # 96 cells: C = 2 and 48 threads per lane, no whole warps, so no outcomes; two lanes per CTA, a ragged last group;
+    # fewer steps than ring stages
+    (301, 96, 2): [
+        ((1, True, False), {"*": ((2, 2, 4, _F, _F, _F), (2, 2, 0, _F, _F, _F))}),
+        ((1, True, True), {"*": ((2, 2, 4, _F, _F, _F), (2, 2, 1, _T, _F, _F))}),
+        ((8, True, False), {"*": ((2, 2, 0, _F, _F, _F), (2, 2, 2, _F, _F, _F))}),
+    ],
+    # 2048 cells: C = 8
+    (40, 2048, 5): [
+        ((1, True, False), {"float64": ((8, 2, 0, _F, _F, _F), (8, 2, 0, _F, _F, _F)),
+                            "float32": ((8, 2, 4, _F, _T, _F), (8, 2, 0, _F, _T, _F))}),
+        ((1, True, True), {"float64": ((8, 2, 0, _F, _F, _F), (8, 2, 1, _T, _F, _F)),
+                           "float32": ((8, 2, 4, _F, _F, _F), (8, 2, 1, _T, _F, _F))}),
+        ((8, True, False), {"*": ((8, 2, 0, _F, _F, _F), (8, 2, 2, _F, _F, _F))}),
+    ],
+    # 10 cells: C = 1, register-prefetch adjoint; 12 lanes per CTA, a ragged last group
+    (301, 10, 9): [
+        ((1, True, False), {"*": ((1, 1, 0, _F, _F, _F), (1, 1, 1, _F, _F, _F))}),
+        ((1, True, True), {"*": ((1, 1, 0, _F, _F, _F), (1, 1, 1, _T, _F, _F))}),
+        ((8, True, False), {"*": ((1, 1, 0, _F, _F, _F), (1, 1, 2, _F, _F, _F))}),
+    ],
+    # 98 cells: C = 2; fp32 rows of 392 bytes take the register-prefetch adjoint
+    (37, 98, 9): [
+        ((1, True, False), {"float64": ((2, 2, 4, _F, _F, _F), (2, 2, 0, _F, _F, _F)),
+                            "float32": ((2, 2, 0, _F, _F, _F), (2, 2, 1, _F, _F, _F))}),
+        ((8, True, False), {"*": ((2, 2, 0, _F, _F, _F), (2, 2, 2, _F, _F, _F))}),
+    ],
+}
+
+
+def _rollout_kernels(prof):
+    """{"fwd" / "bwd": set of template-argument tuples} of the rollout kernels in a profile's CUDA activity."""
+    import re
+    pat = re.compile(r"arz_rollout_(fwd|bwd)_reg_kernel<(?:double|float), (\d+), (\d+), (\d+), (\w+), (\w+), (\w+)>")
+    out = {"fwd": set(), "bwd": set()}
+    for e in prof.events():
+        m = pat.search(e.name)
+        if m and e.device_type == torch.autograd.DeviceType.CUDA:
+            out[m.group(1)].add(tuple(int(x) for x in m.group(2, 3, 4)) + tuple(x == "true" for x in m.group(5, 6, 7)))
+    return out
+
+
 @pytest.mark.parametrize("dtype", [torch.float64, torch.float32])
-def test_rollout_tma_paths_equal_plain_paths(dev, dtype):
-    """Every state stored: the forward's staged TMA bulk stores (shared-memory staging ring, cp.async.bulk to HBM) and
-    the adjoint's TMA state ring (cp.async.bulk into shared memory, mbarrier completion) against the per-thread
-    store / register-prefetch variants.  Same arithmetic, so gradients must agree to rounding (observed: bitwise
-    or 1 ulp) -- persistent loop over more lane groups than CTAs, ragged last group, fewer steps than ring
-    stages, stored-speed first step."""
-    import os
+@pytest.mark.parametrize("shape", list(_ROUTES), ids=lambda s: "B%d_N%d_T%d" % s)
+def test_rollout_routes_agree(dev, dtype, shape):
+    """Every launch route of the fused rollout on the same seeded inputs: the staged forward (TMA bulk stores from a
+    shared-memory staging ring, with and without the stored interface outcomes) or per-thread stores, and the adjoint's TMA
+    state ring, register prefetch (EXT: with the state history) or segment recompute.  The kernels that ran are read from
+    the profiler, so no route can silently fall into another one; the stored-speed first step is part of every route.
+    Same arithmetic, so states and gradients agree to rounding (observed: bitwise or 1 ulp)."""
     import dhts_b200
     from dhts_b200 import functional as F
+    from torch.profiler import ProfilerActivity, profile
+    B, N, T = shape
     rng = np.random.default_rng(5)
-    variants = {"tma": {}, "ring2": {"DHTS_ARZ_RING": "2"}, "plain_adj": {"DHTS_ARZ_RING": "0"},
-                "plain": {"DHTS_ARZ_RING": "0", "DHTS_ARZ_STAGE": "0"}}
-    for B, N, T in ((701, 1024, 7), (301, 64, 9), (9, 256, 2), (40, 2048, 5)):
-        r0 = rng.uniform(0, 1, (B, N)); u0 = rng.uniform(0, 30, (B, N))
-        gr = rng.uniform(0, 1, (B, 2)); gu = rng.uniform(0, 30, (B, 2)); w = rng.normal(size=(B, N))
-        t = lambda a: torch.tensor(a, dtype=dtype, device=dev)
-        out = {}
-        for name, env in variants.items():
-            os.environ.update(env)
-            try:
-                flags = dhts_b200.Flags(dev)
-                tr, tu = t(r0).requires_grad_(), t(u0).requires_grad_()
-                tgr, tgu = t(gr).requires_grad_(), t(gu).requires_grad_()
-                rT, yT, uT = F.arz_rollout(tr, tu, tgr, tgu, 5.0, 30.0, 0.01, T, ckpt_every=1, flags=flags)
-                ((rT * t(w)).sum() + (uT * t(w / 30)).sum()).backward()
-                flags.check()
-                out[name] = [x.clone() for x in (rT.detach(), uT.detach(), tr.grad, tu.grad, tgr.grad, tgu.grad)]
-            finally:
-                for k in env:
-                    del os.environ[k]
-        tol = 1e-13 if dtype == torch.float64 else 1e-5       # same arithmetic; the compiler may contract differently
-        for name in ("tma", "ring2", "plain_adj"):
-            for a, b in zip(out[name], out["plain"]):
-                assert relerr(a.cpu(), b.cpu()) < tol, (B, N, T, name)
+    r0 = rng.uniform(0, 1, (B, N)); u0 = rng.uniform(0, 30, (B, N))
+    gr = rng.uniform(0, 1, (B, 2)); gu = rng.uniform(0, 30, (B, 2)); w = rng.normal(size=(B, N))
+    t = lambda a: torch.tensor(a, dtype=dtype, device=dev)
+    outs = []
+    for (K, uni, hist), want in _ROUTES[shape]:
+        flags = dhts_b200.Flags(dev)
+        tr, tu = t(r0).requires_grad_(), t(u0).requires_grad_()
+        tgr, tgu = t(gr).requires_grad_(), t(gu).requires_grad_()
+        dx, umax = (5.0, 30.0) if uni else (torch.full((B,), 5.0, dtype=dtype, device=dev), torch.full((B,), 30.0, dtype=dtype, device=dev))
+        with profile(activities=[ProfilerActivity.CUDA]) as prof:
+            res = F.arz_rollout(tr, tu, tgr, tgu, dx, umax, 0.01, T, ckpt_every=K, flags=flags, return_history=hist)
+            rT, yT, uT = res[:3]
+            loss = (rT * t(w)).sum() + (uT * t(w / 30)).sum()
+            if hist:
+                loss = loss + (res[3] * 0).sum()
+            loss.backward()
+            torch.cuda.synchronize(dev)
+        flags.check()
+        fwd, bwd = want.get(str(dtype).split(".")[-1], want.get("*"))
+        assert _rollout_kernels(prof) == {"fwd": {fwd}, "bwd": {bwd}}, (K, uni, hist)
+        outs.append([x.detach().clone() for x in (rT, yT, uT, tr.grad, tu.grad, tgr.grad, tgu.grad)])
+    tol = 1e-13 if dtype == torch.float64 else 1e-5       # same arithmetic; the compiler may contract differently
+    for i, o in enumerate(outs[1:], 1):
+        for a, b in zip(o, outs[0]):
+            assert relerr(a.cpu(), b.cpu()) < tol, _ROUTES[shape][i][0]
 
 
 def test_rollout_equals_chained_steps(dev):
