@@ -14,7 +14,7 @@
 // Forward: state checkpoints every K steps to HBM.  Adjoint: segments walked
 // backwards; each is recomputed from its checkpoint while stashing every state
 // in a per-CTA scratch (L2-resident), then the flux-difference adjoint of
-// dhts_arz.cuh is applied step by step, last to first.
+// dhts_arz_lean.cuh is applied step by step, last to first.
 //
 // Replaces T x (RoadNetwork.forward -> dMacroLane.forward -> dMacroForwardLayer)
 // and the autograd chain through them (example/inverse/_inverse.py:91-99,227;
@@ -212,6 +212,8 @@ __device__ __forceinline__ void setup_group(const Shm<T>& s, int lane0, int nl, 
         int l = e >> 1, side = e & 1;
         const T* g = ghost + ((size_t)(lane0 + l) * 2 + side) * 3;          // (r, y, u) built by from_r_u
         const LaneK<T> k = dx ? make_lanek<T>(umax_[lane0 + l], dx[lane0 + l], dt) : kall;
+        // frec_stored / arec_stored with no stored u_eq, spelled out: through them the compiler schedules the fp64 MODE 2,
+        // C = 2 adjoint kernel differently
         FRec<T> f = fderive<T, true>(g[0], g[1], g[2], k);
         if (g[0] < DHTS_EPS) f.w = w_vacuum(g[0], f.us, k);
         pack(f, s.ghostF + (l * 2 + side) * GH_F);
@@ -230,14 +232,10 @@ template <typename T, bool ADJ>
 __device__ __forceinline__ void step_ghost_record(const Shm<T>& s, int e, int lpc, int par, const T* g) {
     const LaneK<T> k = s.lk[e >> 1];
     if (!ADJ) {
-        FRec<T> f = fderive<T, true>(g[0], g[1], g[2], k);
-        if (g[0] < DHTS_EPS) f.w = w_vacuum(g[0], f.us, k);
-        pack(f, s.ghostF + ((size_t)par * lpc * 2 + e) * GH_F);
+        pack(frec_stored<T>(g[0], g[1], g[2], T(0), false, k), s.ghostF + ((size_t)par * lpc * 2 + e) * GH_F);
     } else {
-        ARec<T> a = aderive<T, true>(g[0], g[1], g[2], k);
-        if (g[0] < DHTS_EPS) fix_vacuum_adj(a, g[1], k);
         T tmp[RF_ADJ];
-        pack(a, T(0), T(0), tmp);
+        pack(arec_stored<T>(g[0], g[1], g[2], T(0), false, k), T(0), T(0), tmp);
 #pragma unroll
         for (int i = 0; i < GH_A; i++) s.ghostA[((size_t)par * lpc * 2 + e) * GH_A + i] = tmp[i];
     }

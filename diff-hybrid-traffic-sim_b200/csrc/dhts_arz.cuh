@@ -1,20 +1,11 @@
-// ARZ (Aw-Rascle-Zhang) device math for the B200 path: per-cell derived record,
-// per-interface Riemann flux, per-interface adjoint in flux-difference form.
+// ARZ (Aw-Rascle-Zhang) device primitives shared by every kernel: flags, constants, the branch-free
+// reciprocal / square roots, and the closures u_eq, compute_u and the derivative of compute_u.  The
+// per-cell records, the Riemann solver and its adjoint are in dhts_arz_lean.cuh.
 //
 // Behaviour restated from the reference (file:line relative to its checkout):
 //   model/macro/_arz.py:121-149      u_eq, u_eq', compute_u, compute_y
-//   model/macro/_arz.py:155-199      Q_L / Q_C / Q_M candidate states
-//   model/macro/_arz.py:212-332      riemann_solve case tree (order matters)
-//   model/macro/darz.py:12-233       dL / dM / dC Jacobians and flux_prime
-//   road/lane/_macro_lane.py:83-146  Godunov update and CFL assert
-//   road/lane/dmacro_lane.py:96-132, 277-310  Jacobian band and its VJP
 // gamma is the module constant 0.5 (no caller overrides it), so r^gamma =
 // sqrt(r), r^(gamma-1) = 1/sqrt(r), x^(1/gamma) = x*x.
-//
-// The adjoint is NOT a stored Jacobian band: with A_i = F'(Q0_i) dQ0_i/dQ_left
-// and B_i = F'(Q0_i) dQ0_i/dQ_right per interface i, and w_i = g_{i+1} - g_i,
-//   gbar_j = g_j + c (A_j^T w_j + B_{j-1}^T w_{j-1})           (SURVEY A.3)
-// which is algebraically the band-transpose product of dmacro_lane.py:293-303.
 #pragma once
 #include <cuda_runtime.h>
 
@@ -111,17 +102,6 @@ template <typename T> __device__ __forceinline__ bool t_isnan(T x) { return !(x 
 #define DHTS_EPS_LIT (T(1e-5))
 #define DHTS_RSQRT_EPS_LIT (T(316.22776601683796))
 
-// Per-cell record.  The reference STORES u and u_eq on each cell instead of
-// recomputing them at use (SURVEY App. B.3):
-//   us = stored speed (drives the case tree, Q_M and Q_C),
-//   uc = compute_u(r, y) (what a Q_L outcome re-derives, _arz.py:155-165),
-//   w  = u_max + us - u_eq_stored (every vacuum / rarefaction test, :237,283,308),
-//   uf = u_eq(r) freshly evaluated (what flux_prime sees on Q_L, darz.py:217-233),
-//   sq = sqrt(max(r,eps)), rs = 1/sq, ri = 1/max(r,eps)  (rs, ri: adjoint only).
-template <typename T> struct Cell {
-    T r, y, us, uc, w, sq, rs, ri, uf;
-};
-
 // u_eq(r) = u_max (1 - (max(r,0)+eps)^gamma)                    _arz.py:133-138
 template <typename T> __device__ __forceinline__ T u_eq(T r, T umax) {
     return umax * (T(1) - f_sqrt_pos(t_max(r, T(0)) + DHTS_EPS));      // argument >= eps: branch-free sqrt (<= 1 ulp)
@@ -130,151 +110,6 @@ template <typename T> __device__ __forceinline__ T u_eq(T r, T umax) {
 template <typename T> __device__ __forceinline__ T compute_u(T r, T y, T umax) {
     T rc = t_max(r, DHTS_EPS);
     return y * f_rcp(rc) + umax * (T(1) - f_sqrt_pos(rc + DHTS_EPS));  // rc >= eps: no IEEE division / sqrt slow paths
-}
-
-// Record of a cell whose (u, u_eq) follow set_r_y (_arz.py:88-92), i.e. every
-// interior cell after a step.
-template <typename T, bool ADJ> __device__ __forceinline__ Cell<T> derive_cell(T r, T y, T umax) {
-    Cell<T> c;
-    T rc = t_max(r, DHTS_EPS);
-    T re = rc + DHTS_EPS;
-    T ueq_c = umax * (T(1) - f_sqrt_pos(re));          // compute_u evaluates u_eq at the clamped r
-    c.r = r; c.y = y;
-    c.rs = f_rsqrt(rc);                                // rc^(gamma-1)
-    c.sq = rc * c.rs;                                  // rc^gamma
-    c.ri = c.rs * c.rs;                                // 1/rc
-    c.uc = y * c.ri + ueq_c;
-    c.us = c.uc;
-    // u_eq(r) differs from ueq_c only below eps (max(r,0)+eps vs max(r,eps)+eps)
-    c.uf = (r >= DHTS_EPS) ? ueq_c : umax * (T(1) - f_sqrt_pos(t_max(r, T(0)) + DHTS_EPS));
-    c.w = umax + c.us - c.uf;
-    return c;
-}
-
-// Record of a cell with an explicitly stored speed: ghosts built by from_r_u
-// (_arz.py:74-80), initial cells set by set_r_u (:82-86), cells rewritten by
-// micro_to_macro (conversion.py:157-167; their stored u_eq is stale).
-template <typename T, bool ADJ>
-__device__ __forceinline__ Cell<T> derive_cell_stored(T r, T y, T us, T ueq_stored, bool have_ueq, T umax) {
-    Cell<T> c = derive_cell<T, ADJ>(r, y, umax);
-    c.us = us;
-    c.w = umax + us - (have_ueq ? ueq_stored : c.uf);
-    return c;
-}
-
-template <typename T> struct Riem {
-    int cas;        // 0 = Q_L, 1 = Q_M, 2 = Q_C                 _arz.py:209
-    T r0, y0, u0, ueq0;
-    T rootr;        // sqrt(r0) without re-evaluating a square root (r0 = b^2 for Q_M / Q_C)
-    bool cfl_bad;
-};
-
-// Riemann solve at one interface.  Case tree of _arz.py:225-322, selected state per
-// :324-336, written BRANCH-FREE: with a 86/9/5 % outcome mix nearly every warp holds
-// all three outcomes, so a divergent tree executes every path anyway while blocking
-// instruction-level overlap between the C independent cells of a thread.  Where the
-// reference only consumes the SIGN of a wave speed the division is skipped; the CFL
-// test dt < dx / max(|s|,1e-5) is evaluated as dt * max(|s|,1e-5) < dx.
-template <typename T>
-__device__ __forceinline__ Riem<T> riemann(const Cell<T>& L, const Cell<T>& R, T umax, T inv_umax, T inv15, T dt,
-                                           T dx) {
-    Riem<T> o;
-    const bool vacL = L.r < DHTS_EPS;                              // :225
-    const bool vacR = R.r < DHTS_EPS;                              // :235
-    const T du = L.us - R.us;
-    const bool same = t_abs(du) < DHTS_EPS;                        // :256
-    const bool shock = du > T(0);                                  // :265
-    const bool rare = L.w > R.us;                                  // :283
-    const T lam0l = L.us - T(0.5) * umax * L.sq;                   // u + r u_eq'(r) for r >= eps   :103
-    const T b = L.sq + du * inv_umax;                              // Q_M: r_m = b^2               :194
-    const T rm = b * b;
-    const T fd = rm * R.us - L.r * L.us;                           // :268
-    const T den = t_max(rm - L.r, DHTS_EPS);
-    const T lam0m_r = R.us - T(0.5) * umax * ((rm >= DHTS_EPS) ? t_abs(b) : rm * DHTS_RSQRT_EPS);
-    const T s_vac = (lam0l + L.w) * T(0.5);                        // :247, :315
-    const T s_rare = (lam0l + lam0m_r) * T(0.5);                   // :292
-    const bool l0 = lam0l >= T(0);
-    // outcome index per branch, then the first matching branch wins
-    const int c_vac = l0 ? 0 : 2;
-    const int c_shock = (fd >= T(0)) ? 0 : 1;
-    const int c_rare = l0 ? 0 : ((lam0m_r <= T(0)) ? 1 : 2);
-    const int c_tail = shock ? c_shock : (rare ? c_rare : c_vac);
-    o.cas = vacL ? 0 : (vacR ? c_vac : (same ? 0 : c_tail));
-    // wave speeds for the CFL test (_macro_lane.py:137-146)
-    const bool use_shock = !vacL && !vacR && !same && shock;
-    const T s0 = (vacL || (!vacR && same)) ? T(0) : (vacR ? s_vac : (rare ? s_rare : s_vac));
-    const T s1 = vacL ? L.us : (vacR ? s_vac : R.us);
-    const bool ok1 = dt * t_max(t_abs(s1), T(1e-5)) < dx;
-    const bool ok0s = dt * t_max(t_abs(fd), T(1e-5) * den) < dx * den;
-    const bool ok0n = dt * t_max(t_abs(s0), T(1e-5)) < dx;
-    o.cfl_bad = !((use_shock ? ok0s : ok0n) && ok1);
-    // selected state: Q_L (:155-165), Q_M (:186-199) or Q_C (:168-183)
-    const T sc = L.us + umax * L.sq;
-    const T q = sc * inv15;
-    const bool isL = o.cas == 0, isM = o.cas == 1;
-    const T root = isM ? b : q;
-    o.rootr = isL ? L.sq : t_abs(root);
-    o.r0 = isL ? L.r : root * root;
-    o.u0 = isL ? L.uc : (isM ? R.us : (T(0.5) / T(1.5)) * sc);
-    const T ueq_new = umax * (T(1) - f_sqrt_pos(root * root + DHTS_EPS));
-    o.ueq0 = isL ? L.uf : ueq_new;
-    o.y0 = isL ? L.y : o.r0 * (o.u0 - ueq_new);
-    return o;
-}
-
-// Adjoint of one interface flux: given w = g_{right} - g_{left} (2-vector),
-// returns pa = A^T w (goes to the left cell) and pb = B^T w (right cell).
-// L and R must carry rs / ri (derive_cell<T, true>).
-template <typename T>
-__device__ __forceinline__ void riemann_adj(const Cell<T>& L, const Cell<T>& R, const Riem<T>& s, T umax, T inv_umax,
-                                            T inv15, T wr, T wy, T& par, T& pay, T& pbr, T& pby) {
-    const bool isL = s.cas == 0, isM = s.cas == 1;
-    // flux_prime at Q0 (darz.py:217-233), transposed and applied to w
-    const bool big = s.r0 >= DHTS_EPS;
-    const T rr = t_max(s.r0, DHTS_EPS);
-    const T inv_root = f_rcp(t_max(s.rootr, T(1e-30)));
-    const T inv_sq = isL ? L.rs : (big ? inv_root : DHTS_RSQRT_EPS);
-    const T inv_rr = isL ? L.ri : inv_sq * inv_sq;
-    const T ueqp0 = T(-0.5) * umax * inv_sq;                 // u_eq'(max(r0,eps))  _arz.py:146-149
-    const T yr = s.y0 * inv_rr;
-    const T f00 = s.ueq0 + rr * ueqp0;
-    const T f10 = s.y0 * ueqp0 - yr * yr;
-    const T f11 = T(2) * yr + s.ueq0;
-    const T z0 = f00 * wr + f10 * wy;
-    const T z1 = wr + f11 * wy;
-    // shared pieces of dM (darz.py:35-122) and dC (darz.py:124-192)
-    const T ueqpL = T(-0.5) * umax * L.rs;
-    const T duL_drL = -L.y * L.ri * L.ri + ueqpL;
-    const T duL_dyL = L.ri;
-    const T ueqpR = T(-0.5) * umax * R.rs;
-    const T duR_drR = -R.y * R.ri * R.ri + ueqpR;
-    const T duR_dyR = R.ri;
-    const T a = T(2) * s.rootr;                              // (1/gamma) r0^(1-gamma)
-    const T g = s.u0 - s.ueq0;
-    const T k = g - s.r0 * ueqp0;
-    // Q_M
-    const T drM_drL = a * (T(0.5) * L.rs + duL_drL * inv_umax);
-    const T drM_dyL = a * (duL_dyL * inv_umax);
-    const T drM_drR = -a * (duR_drR * inv_umax);
-    const T drM_dyR = -a * (duR_dyR * inv_umax);
-    const T dyM_drR = drM_drR * k + s.r0 * duR_drR;
-    const T dyM_dyR = drM_dyR * k + s.r0 * duR_dyR;
-    // Q_C
-    const T g13 = T(0.5) / T(1.5);
-    const T f = umax * T(0.5) * L.rs;
-    const T e = a * inv15;                                   // rC^(1-gamma) / gamma / ((gamma+1) u_max)
-    const T drC_drL = e * (duL_drL + f);
-    const T drC_dyL = e * duL_dyL;
-    const T dyC_drL = drC_drL * k + s.r0 * (g13 * (duL_drL + f));
-    const T dyC_dyL = drC_dyL * k + s.r0 * (g13 * duL_dyL);
-    // d Q0 / d Q_left (2x2) and d Q0 / d Q_right, selected by outcome (Q_L: identity / zero, darz.py:12-33)
-    const T d00 = isL ? T(1) : (isM ? drM_drL : drC_drL);
-    const T d01 = isL ? T(0) : (isM ? drM_dyL : drC_dyL);
-    const T d10 = isL ? T(0) : (isM ? drM_drL * k : dyC_drL);
-    const T d11 = isL ? T(1) : (isM ? drM_dyL * k : dyC_dyL);
-    par = d00 * z0 + d10 * z1; pay = d01 * z0 + d11 * z1;
-    pbr = isM ? (drM_drR * z0 + dyM_drR * z1) : T(0);
-    pby = isM ? (drM_dyR * z0 + dyM_dyR * z1) : T(0);
 }
 
 // d compute_u / d(r, y) as autograd differentiates set_r_y OUTSIDE the

@@ -1,8 +1,7 @@
-// Lean ARZ device math for the fused rollouts (arz_rollout.cu): the same step and the
-// same analytic adjoint as dhts_arz.cuh, re-associated so that everything that depends
-// on ONE cell is evaluated once per cell and an interface only does what couples two
-// cells.  fp64 instruction count per cell-step drops from ~93 to ~68 (forward) and from
-// ~140 to ~100 (adjoint) against the straightforward form (profiles/r1d vs r1e).
+// ARZ per-cell records, Riemann solver and its adjoint, for every ARZ kernel: the single step
+// (arz_kernels.cu), the fused lane rollouts (arz_rollout.cu) and the network rollouts (dhts_net_if.cuh).
+// Everything that depends on ONE cell is evaluated once per cell, in its record; an interface only
+// does what couples two cells.
 //
 // Reference behaviour restated (file:line relative to the reference checkout):
 //   model/macro/_arz.py:121-149,155-199,212-332   closures, candidate states, case tree
@@ -11,7 +10,10 @@
 //   road/lane/dmacro_lane.py:96-132,277-310       Jacobian band and its VJP
 //
 // Forward.  The interface flux is selected, not the interface state: for outcome Q_L it is
-// (r uc, y uc) of the left cell (per-cell), otherwise (r0 u0, y0 u0) of Q_M / Q_C.
+// (r uc, y uc) of the left cell (per-cell), otherwise (r0 u0, y0 u0) of Q_M / Q_C.  The case tree
+// is BRANCH-FREE: with a 86/9/5 % outcome mix nearly every warp holds all three outcomes, so a
+// divergent tree executes every path anyway while blocking instruction-level overlap between the
+// independent cells of a thread.
 //
 // CFL.  The reference asserts dt < dx / max(|s|, 1e-5) for two wave speeds per interface
 // (_macro_lane.py:137-146), i.e. |s| < dx/dt =: V.  Every non-shock speed is an average of
@@ -22,10 +24,15 @@
 //   fd / (r_m - r_L) = u_R - r_L u_max / (2 sqrt(r_L) + du/u_max),   |.| <= |u_R| + (u_max/2) sqrt(r_L) < V/2,
 // and clamping the denominator up to eps only shrinks |s|: the same two per-cell tests cover it.
 // Only when one of these SUFFICIENT tests fails (never in a run the reference would accept) is the
-// exact per-branch evaluation done (cfl_exact_bad).
+// exact per-branch evaluation done (cfl_exact_bad; it evaluates dt < dx / max(|s|, 1e-5) as
+// dt * max(|s|, 1e-5) < dx, with no division).
 //
-// Adjoint.  With z = F'(Q0)^T w, k = (u0 - u_eq0) - r0 u_eq'(r0), s = z0 + k z1 and
-// a = 2 sqrt(r0), the products dQ0/dQ_L^T z and dQ0/dQ_R^T z of darz.py collapse to
+// Adjoint.  Not a stored Jacobian band: with A_i = F'(Q0_i) dQ0_i/dQ_left and
+// B_i = F'(Q0_i) dQ0_i/dQ_right per interface i, and w_i = g_{i+1} - g_i,
+//   gbar_j = g_j + c (A_j^T w_j + B_{j-1}^T w_{j-1})           (SURVEY A.3)
+// which is algebraically the band-transpose product of dmacro_lane.py:293-303.  With
+// z = F'(Q0)^T w, k = (u0 - u_eq0) - r0 u_eq'(r0), s = z0 + k z1 and a = 2 sqrt(r0), the
+// products dQ0/dQ_L^T z and dQ0/dQ_R^T z of darz.py collapse to
 //   Q_L:  A^T w = F'(cell L)^T w                       B^T w = 0
 //   Q_M:  A^T w = (s a / u_max) P_L                    B^T w = (r0 z1 - s a / u_max) D_R
 //   Q_C:  A^T w = (s a / (1.5 u_max) + r0 z1 / 3) P_L  B^T w = 0
@@ -100,6 +107,16 @@ __device__ __forceinline__ FRec<T> fderive(T r, T y, T us_in, const LaneK<T>& k)
 template <typename T> __device__ __forceinline__ T w_vacuum(T r, T us, const LaneK<T>& k) {
     return fma(-k.umax, T(1) - f_sqrt_pos(t_max(r, T(0)) + DHTS_EPS), k.umax + us);
 }
+// Record of a cell with an explicitly stored speed us, vacuum fix-up included: ghosts built by from_r_u (_arz.py:74-80),
+// cells set by set_r_u (:82-86), network cells (nu = compute_u(nr, ny) is stored).  have_ueq: the cell also carries a
+// stored u_eq, which then enters w (stale on cells a micro->macro deposit rewrote, conversion.py:157-167).
+template <typename T>
+__device__ __forceinline__ FRec<T> frec_stored(T r, T y, T us, T ueq_stored, bool have_ueq, const LaneK<T>& k) {
+    FRec<T> f = fderive<T, true>(r, y, us, k);
+    if (have_ueq) f.w = k.umax + us - ueq_stored;
+    else if (r < DHTS_EPS) f.w = w_vacuum(r, us, k);
+    return f;
+}
 
 // Outcome predicates of the case tree (_arz.py:225-322), shared by forward and adjoint.
 template <typename T> struct Tree { bool isL, isM, shock; T b, sc, q, rm, fd; };
@@ -151,20 +168,9 @@ __device__ __forceinline__ bool cfl_exact_bad(T Lr, T Lus, T Lsq, T Lw, T Rr, T 
     return !((use_shock ? ok0s : ok0n) && ok1);
 }
 
-// Flux through the interface between cell L (record) and a right cell (r, stored speed).
-template <typename T, bool VAC = true>
-__device__ __forceinline__ void fflux(const FRec<T>& L, T Rr, T Rus, const LaneK<T>& k, T& fr, T& fy) {
-    const Tree<T> t = case_tree<T, VAC>(L.r, L.us, L.sq, L.w, Rr, Rus, k);
-    const T root = t.isM ? t.b : t.q;
-    const T r0 = root * root;
-    const T u0 = t.isM ? Rus : t.sc * KC<T>::third();
-    const T ueq = fma(-k.umax, f_sqrt_pos(fma(root, root, DHTS_EPS)), k.umax);
-    const T y0 = r0 * (u0 - ueq);
-    fr = t.isL ? L.fr : r0 * u0;
-    fy = t.isL ? L.fy : y0 * u0;
-}
-
-// Stored interface outcome (forward -> adjoint through HBM): two bits per interface and step (Q_L, Q_M).  With them the
+// Flux through the interface between cell L (record) and a right cell (r, stored speed), and the interface's outcome
+// (Q_L, Q_M; neither: Q_C).
+// The rollouts store the outcome (forward -> adjoint through HBM): two bits per interface and step.  With them the
 // adjoint skips the case tree.  (Storing sqrt(r0 + eps) of the selected state as well -- 8 bytes per cell-step, so that the
 // adjoint skips that square root too -- was measured: adjoint 629 -> 580 ms per pass but forward 381 -> 411 ms, the forward
 // kernel does not take 24 instead of 16 bytes of writes per cell-step for free.)
@@ -179,6 +185,11 @@ __device__ __forceinline__ void fflux_x(const FRec<T>& L, T Rr, T Rus, const Lan
     fr = t.isL ? L.fr : r0 * u0;
     fy = t.isL ? L.fy : y0 * u0;
     isL = t.isL; isM = t.isM;
+}
+template <typename T, bool VAC = true>
+__device__ __forceinline__ void fflux(const FRec<T>& L, T Rr, T Rus, const LaneK<T>& k, T& fr, T& fy) {
+    bool isL, isM;
+    fflux_x<T, VAC>(L, Rr, Rus, k, fr, fy, isL, isM);
 }
 
 // ---------------------------------------------------------------------------- adjoint
@@ -224,56 +235,21 @@ template <typename T> __device__ __forceinline__ void fix_vacuum_adj(ARec<T>& c,
     c.f00 = fma(DHTS_EPS_LIT, c.ueqp, uf);
     c.f11 = fma(T(2), y * c.ri, uf);
 }
-
-// A^T w -> (par, pay) for the left cell, B^T w -> (pbr, pby) for the right cell (see header).
-template <typename T, bool VAC = true>
-__device__ __forceinline__ void aflux(const ARec<T>& L, const ARec<T>& R, T wr, T wy, const LaneK<T>& k, T& par,
-                                      T& pay, T& pbr, T& pby) {
-    const Tree<T> t = case_tree<T, VAC>(L.r, L.us, L.sq, L.w, R.r, R.us, k);
-    const T root = t.isM ? t.b : t.q;
-    const T r0 = root * root;
-    const T rootr = t_abs(root);
-    const T u0 = t.isM ? R.us : t.sc * (T(0.5) / T(1.5));
-    const T ueq0 = fma(-k.umax, f_sqrt_pos(fma(root, root, DHTS_EPS_LIT)), k.umax);
-    const T g = u0 - ueq0;
-    const T y0 = r0 * g;
-    // flux_prime at Q0 with r clamped at eps
-    // flux_prime at Q0 clamps r at eps: with rootc = sqrt(max(r0, eps)) both clamped quantities follow without a select on
-    // constants (1 / sqrt(max(r0, eps)) and max(r0, eps); at r0 < eps they differ from the literal 1 / sqrt(eps), eps by an ulp)
-    const T rootc = t_max(rootr, KC<T>::sqrt_eps());
-    const T inv_sq = f_rcp(rootc);
-    const T rr = rootc * rootc;
-    const T ueqp0 = -k.hum * inv_sq;
-    const T yr = y0 * (inv_sq * inv_sq);
-    const T f00 = fma(rr, ueqp0, ueq0);
-    const T f10 = fma(y0, ueqp0, -(yr * yr));
-    const T f11 = fma(T(2), yr, ueq0);
-    const T z0 = fma(f10, wy, f00 * wr);
-    const T z1 = fma(f11, wy, wr);
-    const T kk = fma(-r0, ueqp0, g);
-    const T s = fma(kk, z1, z0);
-    const T sa = s * (T(2) * rootr);
-    const T cM = sa * k.inv_umax;
-    const T r0z1 = r0 * z1;
-    const T cC = fma(sa, k.inv15, r0z1 * (T(0.5) / T(1.5)));
-    const T coef = t.isM ? cM : cC;
-    // outcome Q_L: dQ0/dQ_L = I
-    const T zl0 = fma(L.f10, wy, L.f00 * wr);
-    const T zl1 = fma(L.f11, wy, wr);
-    par = t.isL ? zl0 : coef * L.plr;
-    pay = t.isL ? zl1 : coef * L.ri;
-    const T cB = t.isM ? (r0z1 - cM) : T(0);
-    pbr = cB * (R.plr + R.ueqp);
-    pby = cB * R.ri;
+// the adjoint record of frec_stored
+template <typename T>
+__device__ __forceinline__ ARec<T> arec_stored(T r, T y, T us, T ueq_stored, bool have_ueq, const LaneK<T>& k) {
+    ARec<T> c = aderive<T, true>(r, y, us, k);
+    if (r < DHTS_EPS) fix_vacuum_adj(c, y, k);
+    if (have_ueq) c.w = k.umax + us - ueq_stored;
+    return c;
 }
 
-// aflux with the interface's outcome stored by the forward pass (fflux_x): no case tree.
-// Uses us, sq, f00, f10, f11, plr, ri of L and us, plr, ri, ueqp of R.
+// A^T w -> (par, pay) for the left cell, B^T w -> (pbr, pby) for the right cell (see header), given the interface's outcome
+// and the roots of its Q_M / Q_C candidates (b and sc of case_tree).  Uses us, sq, f00, f10, f11, plr, ri of L and us, plr,
+// ri, ueqp of R.
 template <typename T>
-__device__ __forceinline__ void aflux_x(const ARec<T>& L, const ARec<T>& R, T wr, T wy, const LaneK<T>& k, bool isL, bool isM,
-                                        T& par, T& pay, T& pbr, T& pby) {
-    const T b = fma(L.us - R.us, k.inv_umax, L.sq);                // Q_M: r_m = b^2
-    const T sc = fma(k.umax, L.sq, L.us);                          // Q_C: r_c = q^2, u_c = sc / 3
+__device__ __forceinline__ void aflux_o(const ARec<T>& L, const ARec<T>& R, T wr, T wy, const LaneK<T>& k, bool isL, bool isM,
+                                        T b, T sc, T& par, T& pay, T& pbr, T& pby) {
     const T root = isM ? b : sc * k.inv15;
     const T r0 = root * root;
     const T rootr = t_abs(root);
@@ -307,6 +283,20 @@ __device__ __forceinline__ void aflux_x(const ARec<T>& L, const ARec<T>& R, T wr
     const T cB = isM ? (r0z1 - cM) : T(0);
     pbr = cB * (R.plr + R.ueqp);
     pby = cB * R.ri;
+}
+template <typename T, bool VAC = true>
+__device__ __forceinline__ void aflux(const ARec<T>& L, const ARec<T>& R, T wr, T wy, const LaneK<T>& k, T& par,
+                                      T& pay, T& pbr, T& pby) {
+    const Tree<T> t = case_tree<T, VAC>(L.r, L.us, L.sq, L.w, R.r, R.us, k);
+    aflux_o<T>(L, R, wr, wy, k, t.isL, t.isM, t.b, t.sc, par, pay, pbr, pby);
+}
+// the same with the outcome the forward pass stored (fflux_x): no case tree
+template <typename T>
+__device__ __forceinline__ void aflux_x(const ARec<T>& L, const ARec<T>& R, T wr, T wy, const LaneK<T>& k, bool isL, bool isM,
+                                        T& par, T& pay, T& pbr, T& pby) {
+    const T b = fma(L.us - R.us, k.inv_umax, L.sq);                // Q_M: r_m = b^2
+    const T sc = fma(k.umax, L.sq, L.us);                          // Q_C: r_c = q^2, u_c = sc / 3
+    aflux_o<T>(L, R, wr, wy, k, isL, isM, b, sc, par, pay, pbr, pby);
 }
 // the mailbox record of that path: the 7 fields aflux_x reads of its LEFT cell + that cell's old adjoint
 constexpr int RF_ADJX = 9;

@@ -95,10 +95,4 @@ __device__ __forceinline__ Side<T> resolve_side(const NetArgs<T>& a, int l, int 
     return o;
 }
 
-// ghost record of from_r_u(r, u): y = r (u - u_eq(r)), stored speed u, fresh u_eq
-template <typename T, bool ADJ> __device__ __forceinline__ Cell<T> ghost_cell(T r, T u, T umax) {
-    const T y = r * (u - u_eq(r, umax));
-    return derive_cell_stored<T, ADJ>(r, y, u, T(0), false, umax);
-}
-
 }  // namespace dhts

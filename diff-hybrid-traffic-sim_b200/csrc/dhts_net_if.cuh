@@ -72,22 +72,6 @@ template <typename T> __device__ __forceinline__ void net_tabs_init(const NetArg
     __syncthreads();
 }
 
-// forward record of a cell with a stored speed (every network cell: nu = compute_u(nr, ny) is STORED, ghosts come from
-// from_r_u, _arz.py:74-92).  have_ueq: the cell also carries a stored u_eq (hybrid networks: stale on cells a
-// micro->macro deposit rewrote, conversion.py:157-167)
-template <typename T> __device__ __forceinline__ FRec<T> net_frec(T r, T y, T us, T ueq_stored, bool have_ueq, const LaneK<T>& k) {
-    FRec<T> f = fderive<T, true>(r, y, us, k);
-    if (have_ueq) f.w = k.umax + us - ueq_stored;
-    else if (r < DHTS_EPS) f.w = w_vacuum(r, us, k);
-    return f;
-}
-template <typename T> __device__ __forceinline__ ARec<T> net_arec(T r, T y, T us, T ueq_stored, bool have_ueq, const LaneK<T>& k) {
-    ARec<T> c = aderive<T, true>(r, y, us, k);
-    if (r < DHTS_EPS) fix_vacuum_adj(c, y, k);
-    if (have_ueq) c.w = k.umax + us - ueq_stored;
-    return c;
-}
-
 // ---------------------------------------------------------------------------------------------- forward, phase I
 // gh [2][L][2]: final ghost (r, u) per (side, lane).  ce: stored u_eq per cell or null.  flux [NI][2].
 // Returns true when the CFL condition (_macro_lane.py:137-146) fails at one of this thread's interfaces.  The exact
@@ -104,10 +88,10 @@ __device__ __forceinline__ bool net_fwd_flux(const NetArgs<T>& a, const NetTabs<
         FRec<T> L;
         if (i == 0) {
             const T gr = gh[2 * l], gu = gh[2 * l + 1];
-            L = net_frec<T>(gr, gr * (gu - u_eq(gr, a.umax)), gu, T(0), false, k);        // from_r_u, _arz.py:74-80
+            L = frec_stored<T>(gr, gr * (gu - u_eq(gr, a.umax)), gu, T(0), false, k);        // from_r_u, _arz.py:74-80
         } else {
             const int c = c0 + i - 1;
-            L = net_frec<T>(cr[c], cy[c], cu[c], ce ? ce[c] : T(0), ce != nullptr, k);
+            L = frec_stored<T>(cr[c], cy[c], cu[c], ce ? ce[c] : T(0), ce != nullptr, k);
         }
         const T Rr = i == N ? gh[2 * (a.L + l)] : cr[c0 + i], Rus = i == N ? gh[2 * (a.L + l) + 1] : cu[c0 + i];
         bad |= cfl_exact_bad(L.r, L.us, L.sq, L.w, Rr, Rus, k, a.dt);
@@ -132,18 +116,18 @@ __device__ __forceinline__ void net_adj_flux(const NetArgs<T>& a, const NetTabs<
         T gLr = T(0), gLy = T(0), gRr = T(0), gRy = T(0);
         if (i == 0) {
             const T gr = gh[2 * l], gu = gh[2 * l + 1];
-            L = net_arec<T>(gr, gr * (gu - u_eq(gr, a.umax)), gu, T(0), false, k);
+            L = arec_stored<T>(gr, gr * (gu - u_eq(gr, a.umax)), gu, T(0), false, k);
         } else {
             const int c = c0 + i - 1;
-            L = net_arec<T>(cr[c], cy[c], cu[c], ce ? ce[c] : T(0), ce != nullptr, k);
+            L = arec_stored<T>(cr[c], cy[c], cu[c], ce ? ce[c] : T(0), ce != nullptr, k);
             gLr = Gr[c]; gLy = Gy[c];
         }
         if (i == N) {
             const T gr = gh[2 * (a.L + l)], gu = gh[2 * (a.L + l) + 1];
-            R = net_arec<T>(gr, gr * (gu - u_eq(gr, a.umax)), gu, T(0), false, k);
+            R = arec_stored<T>(gr, gr * (gu - u_eq(gr, a.umax)), gu, T(0), false, k);
         } else {
             const int c = c0 + i;
-            R = net_arec<T>(cr[c], cy[c], cu[c], ce ? ce[c] : T(0), ce != nullptr, k);
+            R = arec_stored<T>(cr[c], cy[c], cu[c], ce ? ce[c] : T(0), ce != nullptr, k);
             gRr = Gr[c]; gRy = Gy[c];
         }
         T par, pay, pbr, pby;

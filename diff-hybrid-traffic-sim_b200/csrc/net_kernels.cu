@@ -14,7 +14,7 @@
 // Shape of the work: a network is L lanes of a few cells each (ITSCP: 144 lanes of 1-4 cells), coupled every step
 // through ghost cells; replicas (scenarios, candidate signal plans) are independent.  One CTA steps one replica:
 // the whole network state lives in shared memory for the T steps, one thread per lane (its cells are swept
-// serially with the same per-interface math as the lane kernels, dhts_arz.cuh), one block barrier per step.
+// serially with the same per-interface math as the lane kernels, dhts_arz_lean.cuh), one block barrier per step.
 // Long lanes belong to the lane-batched rollout (arz_rollout.cu); this kernel is for many short coupled lanes.
 //
 // Ghost cells.  side 0 = left (upstream), 1 = right.  green = (r, u) of the source; the ITSCP blend is

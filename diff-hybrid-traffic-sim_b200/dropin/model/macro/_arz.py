@@ -5,7 +5,7 @@ Only what callers of the reference touch lives here: the per-cell record ``ARZ.F
 accept Python floats or tensors (any shape, any device) and are differentiated by autograd
 with the TRUE derivative, as the reference's 0-dim tensor arithmetic is.  The Riemann solver
 and its Jacobians (_arz.py:155-332, darz.py) are NOT here: they run inside the CUDA kernels
-(diff-hybrid-traffic-sim_b200/csrc/dhts_arz.cuh).
+(diff-hybrid-traffic-sim_b200/csrc/dhts_arz_lean.cuh).
 """
 import math
 

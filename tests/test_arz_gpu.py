@@ -57,14 +57,22 @@ def test_step_vs_golden_fp32(dev):
 
 
 def test_step_tiles_and_shapes(dev):
-    """Lanes longer than one tile, 1-cell lanes, ragged tile tails: tiled kernel == oracle, fwd and bwd."""
+    """Lanes longer than one tile, 1-cell lanes, ragged tile tails: tiled kernel == oracle, fwd and bwd.  The `vac`
+    shapes put cells and ghosts at r = 0, 5e-6 and exactly eps = 1e-5 (the vacuum branches of the case tree and the
+    records' vacuum fix-ups)."""
     import dhts_b200
     from dhts_b200 import functional as F
     from oracle import oracle as O
     rng = np.random.default_rng(5)
-    for B, N in ((1, 1), (3, 2), (2, 255), (2, 256), (2, 257), (1, 700)):
+    vac_r = np.array([0.0, 5e-6, 1e-5])
+    for B, N, vac in ((1, 1, False), (3, 2, False), (2, 255, False), (2, 256, False), (2, 257, False), (1, 700, False),
+                      (3, 1, True), (3, 5, True), (3, 257, True)):
         dx, umax, dt = 5.0, 30.0, 0.01
         r = rng.uniform(0, 1, (B, N + 2)); u = rng.uniform(0, 1, (B, N + 2)) * umax
+        if vac:
+            m = rng.random((B, N + 2)) < 0.3
+            r[m] = rng.choice(vac_r, m.sum())
+            r[:, 0] = vac_r[np.arange(B) % 3]; r[:, -1] = vac_r[(np.arange(B) + 1) % 3]
         y = O.compute_y(r, u, umax); ue = O.u_eq(r, umax)
         gnr = rng.normal(size=(B, N)); gny = rng.normal(size=(B, N)); gnu = rng.normal(size=(B, N))
         flags = dhts_b200.Flags(dev)
@@ -83,6 +91,56 @@ def test_step_tiles_and_shapes(dev):
                     dy[j] = 1 / eps
             gr, gy = O.arz_vjp(o["dqs"], gnr[b] + gnu[b] * dr, gny[b] + gnu[b] * dy)
             assert relerr(r_pad.grad[b].cpu(), gr) < 1e-10 and relerr(y_pad.grad[b].cpu(), gy) < 1e-10
+        flags.check()
+
+
+@pytest.mark.parametrize("dt", [0.1, 0.01])
+def test_step_cfl_with_stale_stored_ueq(dev, dt):
+    """Dense cells whose stored u_eq is stale (near u_max, as after a micro->macro deposit): |u| and u_max + u - u_eq are
+    both small, yet the rarefaction speed of the middle interface is about -14.4.  With dx = 1 the CFL assert fires at
+    dt = 0.1 (dx / dt = 10) and not at dt = 0.01; the step kernel's flag must follow the oracle."""
+    import dhts_b200
+    from dhts_b200 import functional as F
+    from oracle import oracle as O
+    r = np.array([1.0, 1.0, 1.0, 1.0]); u = np.array([1.0, 1.0, 0.5, 0.5]); ue = np.full(4, 30.0)
+    y = r * (u - ue)
+    o = O.arz_step(r, y, u, ue, 1.0, 30.0, dt)
+    assert o["cfl"] == (dt == 0.1)
+    flags = dhts_b200.Flags(dev)
+    nr, ny, nu = F.arz_step(T64(r[None], dev), T64(y[None], dev), T64(u[None], dev), 1.0, 30.0, dt, flags,
+                            ueq_pad=T64(ue[None], dev))
+    assert bool(flags.read()[0] & dhts_b200._lib.FLAG_CFL) == bool(o["cfl"])
+    assert relerr(nr[0].cpu(), o["nr"]) < 1e-12 and relerr(ny[0].cpu(), o["ny"]) < 1e-12
+
+
+@pytest.mark.parametrize("dtype", [torch.float64, torch.float32])
+def test_step_equals_first_rollout_step_bitwise(dev, dtype):
+    """The single step without a stored u_eq and a one-step rollout, from the same cells (stored speeds) and ghosts,
+    run the same records and interface math: nr, ny, nu agree bit for bit.  N = 37, 50: C = 1 cell per thread; 66: C = 2;
+    128, 1000: C = 4; 2048: C = 8.  Lane 1 has cells and ghosts at and below eps.  Without gradients the rollout stores
+    nothing; with them it runs the staged kernel (C > 1)."""
+    import dhts_b200
+    from dhts_b200 import functional as F
+    rng = np.random.default_rng(17)
+    B, dt = 3, 0.01
+    t = lambda a: torch.tensor(np.asarray(a), dtype=dtype, device=dev)
+    dx, umax = t([5.0, 4.0, 6.0]), t([30.0, 25.0, 35.0])
+    for N in (37, 50, 66, 128, 1000, 2048):
+        r = rng.uniform(0, 1, (B, N + 2)); u = rng.uniform(0, 1, (B, N + 2)) * umax.cpu().numpy()[:, None]
+        m = rng.random(N + 2) < 0.3
+        r[1, m] = rng.choice([0.0, 5e-6, 1e-5], m.sum())
+        r[1, 0], r[1, -1] = 0.0, 5e-6
+        r_pad, u_pad = t(r), t(u)
+        y_pad = F.compute_y(r_pad, u_pad, umax[:, None])
+        ghost = torch.stack([torch.stack([r_pad[:, s], y_pad[:, s], u_pad[:, s]], -1) for s in (0, -1)], 1)
+        flags = dhts_b200.Flags(dev)
+        step = F.arz_step(r_pad, y_pad, u_pad, dx, umax, dt, flags)
+        for grad in (False, True):
+            r0 = r_pad[:, 1:-1].clone().requires_grad_(grad)
+            roll = F.arz_rollout_state(r0, y_pad[:, 1:-1].contiguous(), u_pad[:, 1:-1].contiguous(), ghost, dx, umax, dt,
+                                       1, 1, flags)
+            for name, a, b in zip(("nr", "ny", "nu"), step, roll):
+                assert torch.equal(a, b.detach()), (N, grad, name, (a - b).abs().max().item())
         flags.check()
 
 
